@@ -23,8 +23,13 @@ decoded strings, log-likelihoods and statuses are gathered to rank 0 in input or
 `--impl reference` times the UNMODIFIED reference CPU implementation (oracle/_ref, built from /root/reference by
 oracle/Makefile) on all host cores, one process per core, same metric/config; it composes the machine with the
 reference's own code (refdriver compose) and never imports this repository's library.
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned for its last step as DIR/<name>.npy
+(float64 stays float64, everything else becomes float32). The inputs depend only on the arguments, so two builds can
+be compared output for output.
 """
 import argparse
+import atexit
 import gzip
 import json
 import os
@@ -76,6 +81,31 @@ def cells_of(n_states, k, read_len):
     return int(n_states) * int(np.sum(np.asarray(read_len).astype(np.int64) + 1)) * (k + 2)
 
 
+DUMP_BYTES = 60 << 20  # array data; with the .npy headers a dump stays under 64 MB (64e6 bytes)
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: arrays (name -> array whose first axis is the read / alignment) as <directory>/<name>.npy, plus
+    index.npy, the row numbers written. All rows if they fit in DUMP_BYTES, else a fixed, seeded sample of rows."""
+    n = len(next(iter(arrays.values())))
+    out_dtype = {k: np.float64 if a.dtype == np.float64 else np.float32 for k, a in arrays.items()}
+    row_bytes = 8 + sum(np.dtype(out_dtype[k]).itemsize * int(np.prod(a.shape[1:])) for k, a in arrays.items())
+    m = min(n, DUMP_BYTES // row_bytes)
+    index = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, size=m, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "index.npy"), index.astype(np.float64))
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a[index].astype(out_dtype[k]))
+
+
+def decoded_matrix(strings):
+    """Decoded strings as one byte code per symbol, zero-padded to the longest: [n, max length] uint8."""
+    mat = np.zeros((len(strings), max((len(s) for s in strings), default=0)), dtype=np.uint8)
+    for i, s in enumerate(strings):
+        mat[i, :len(s)] = np.frombuffer(s.encode("latin1"), dtype=np.uint8)
+    return mat
+
+
 class ClockSampler:
     QUERY = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
              "clocks_event_reasons.hw_thermal_slowdown,clocks_event_reasons.sw_thermal_slowdown,"
@@ -90,6 +120,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.QUERY}", "--format=csv,noheader,nounits",
                                           "-i", str(self.device), "-lms", "200"], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.kill)  # never outlive the benchmark, even when it fails before stop()
             self.thread = threading.Thread(target=self._pump, daemon=True)
             self.thread.start()
         except OSError:
@@ -300,6 +331,8 @@ def bench_fwdback(args, w, compiled, dec, rank, local_rank, world, dev, dist, to
     barrier()
     wall_s = time.perf_counter() - t0
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     vals = torch.tensor([kernel_ms, wall_s], dtype=torch.float64, device=dev)
     sums = torch.tensor([float(cells), float(rps * args.steps)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -417,12 +450,13 @@ def short_fwdback(d, util, n_reads=296):
                 max_abs_loglike_back_minus_forward=float(np.abs(out["loglike_back"] - out["loglike"]).max()))
 
 
-def short_pairhmm(d, n_distinct=8192, copies=16, seed=77):
+def short_pairhmm(d, n_distinct=8192, copies=16, seed=77, steps=1, warmup=1, dump=None):
     """Batched pair-HMM forward + backward + expected counts (SURVEY.md 8a-11 / 8f-2) on synthetic alignments:
     reference-encoded ~200-nt strands mutated by the errdecode.pl simulator with the alignment kept
     (benchdata/synth.mutate_aligned), n_distinct alignments repeated `copies` times (the kernel deals alignments to warps in
     order of length, so a warp of 32 holds at least 32 / copies different alignments). DP cells = envelope cells x (2 + k);
-    16 algorithmic bytes per DP cell (the forward cell is written once and read once by the counts pass)."""
+    16 algorithmic bytes per DP cell (the forward cell is written once and read once by the counts pass). `warmup`
+    untimed calls on the distinct alignments, then `steps` timed calls on the whole batch."""
     from benchdata import synth
     rng = np.random.default_rng(seed)
     pool = synth.load_pool("cfg1_l4c4_200b")
@@ -443,11 +477,17 @@ def short_pairhmm(d, n_distinct=8192, copies=16, seed=77):
     for tin, tout, ea, eb in base:
         cells += int((np.abs(ea[:, None] - eb[None, :]) <= k).sum())
     cells *= copies * (2 + k)
-    d.pairhmm_fb_batch(params, base, strict=False)  # warm-up
-    fwd, back, _counts, ms = d.pairhmm_fb_batch(params, aligns, strict=False)
+    for _ in range(warmup):
+        d.pairhmm_fb_batch(params, base, strict=False)
+    ms = 0.0  # mean kernel time of a timed call
+    for _ in range(steps):
+        fwd, back, counts, step_ms = d.pairhmm_fb_batch(params, aligns, strict=False)
+        ms += step_ms / steps
+    if dump:
+        dump_outputs(dump, dict(fwd=fwd, back=back, counts=np.array([c.flat() for c in counts])))
     peak, _ = measured_peak()
     return dict(workload=f"pair-HMM forward + backward + expected counts, {len(aligns)} alignments ({len(base)} distinct) of ~200-nt strands, k = {k}, banded envelope",
-                alignments=len(aligns), dp_cells=cells, kernel_ms=ms, alignments_per_sec=len(aligns) / (ms * 1e-3),
+                alignments=len(aligns), steps=steps, dp_cells=cells, kernel_ms=ms, alignments_per_sec=len(aligns) / (ms * 1e-3),
                 cells_per_sec=cells / (ms * 1e-3), roofline_frac=16.0 * cells / (ms * 1e-3) / 1e9 / peak, kernel="pairHmmFwdBackKernel",
                 max_abs_back_minus_fwd=float(np.abs(np.asarray(fwd) - np.asarray(back)).max()))
 
@@ -466,7 +506,11 @@ def main():
     ap.add_argument("--no-indel", action="store_true", help="decode with --error-del-open 0 --error-dup-prob 0 (closure degenerates)")
     ap.add_argument("--mode", default="viterbi", choices=["viterbi", "fwdback", "pairhmm"],
                     help="fwdback: forward + backward + posterior counts over the machine lattice (weak scaling, one batch per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -489,7 +533,8 @@ def main():
     if args.mode == "pairhmm":
         if rank == 0:
             import dnastore_b200 as d
-            print(json.dumps(short_pairhmm(d, copies=max(1, args.reads_per_step // 8192) if args.reads_per_step else 16)), flush=True)
+            print(json.dumps(short_pairhmm(d, copies=max(1, args.reads_per_step // 8192) if args.reads_per_step else 16,
+                                           steps=args.steps, warmup=args.warmup, dump=args.dump_outputs)), flush=True)
         return
     import torch
     import torch.distributed as dist
@@ -599,7 +644,7 @@ def main():
         parts_ll = g_ll if world > 1 else [d_ll]
         parts_dec = g_dec if world > 1 else [d_dec]
         parts_meta = g_meta if world > 1 else [d_meta]
-        gathered_dec, gathered_ll = [], []
+        gathered_dec, gathered_ll, gathered_status = [], [], []
         for r in range(world):
             n_r = int(cuts[r + 1] - cuts[r])
             ll = parts_ll[r][:n_r].cpu().numpy()
@@ -607,6 +652,11 @@ def main():
             raw = parts_dec[r][:n_r * stride].cpu().numpy().reshape(n_r, stride)
             gathered_ll.extend(ll.tolist())
             gathered_dec.extend(bytes(raw[i, :dl[i]]).decode("latin1") for i in range(n_r))
+            gathered_status.extend(parts_meta[r][shard_max:shard_max + n_r].cpu().numpy().tolist())
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dict(loglike=np.array(gathered_ll, dtype=np.float64), status=np.array(gathered_status),
+                                                 decoded_len=np.array([len(s) for s in gathered_dec]),
+                                                 decoded=decoded_matrix(gathered_dec)))
 
     # ---- e2e: the product's multi-GPU entry on rank 0 over all N devices, host buffers, every step ---------------
     del dev_batches
@@ -739,4 +789,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the tree may be read-only; the benchmark writes nothing there
     main()
