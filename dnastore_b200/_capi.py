@@ -147,7 +147,6 @@ _sig("dnab_decoder_create", _vp, C.POINTER(Tables), C.c_int)
 _sig("dnab_decoder_destroy", None, _vp)
 _sig("dnab_decoder_get_info", C.c_int, _vp, C.POINTER(DecoderInfo))
 _sig("dnab_decoder_configure", C.c_int, _vp, C.c_uint32, C.c_uint32, C.c_uint32)
-_sig("dnab_decoder_configure_ex", C.c_int, _vp, C.c_uint32, C.c_uint32)
 _sig("dnab_decoder_get_stats", C.c_int, _vp, C.POINTER(DecoderStats))
 _sig("dnab_decoder_set_timing", C.c_int, _vp, C.c_int)
 _sig("dnab_decoder_reset_timing", C.c_int, _vp)
@@ -518,16 +517,14 @@ class Decoder:
         self._h = h
         self.device = int(device)
 
-    def configure(self, cluster_size=0, threads_per_cta=0, t_in_smem_mode=0, table_mode=0, partition_mode=0):
+    def configure(self, cluster_size=0, threads_per_cta=0, t_in_smem_mode=0):
+        """Placement overrides of the push kernel (0 = automatic); set_option has the others ("table", "s_prev", ...)."""
         rc = lib.dnab_decoder_configure(self._h, cluster_size, threads_per_cta, t_in_smem_mode)
-        if rc:
-            raise _err(rc)
-        rc = lib.dnab_decoder_configure_ex(self._h, table_mode, partition_mode)
         if rc:
             raise _err(rc)
 
     def set_option(self, key, value):
-        """Named option (include/dnastore_b200.h dnab_decoder_set_option), e.g. kernel=1 (read-batched), 2 (push), 3 (pull)."""
+        """Named option (include/dnastore_b200.h dnab_decoder_set_option), e.g. kernel=1 (read-batched), 2 (push)."""
         rc = lib.dnab_decoder_set_option(self._h, key.encode(), int(value))
         if rc:
             raise _err(rc)

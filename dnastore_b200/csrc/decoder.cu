@@ -51,9 +51,10 @@ struct DevBuf {
   }
 };
 
+// plan of the push kernel (viterbi_fill_push.cu)
 struct LaunchPlan {
-  uint32_t C = 0, M = 0, threads = 0, tInSmem = 0, blocksInSmem = 0, sPrevGlobal = 0, sliceWords = 0, smemBytes = 0, nClusters = 0;
-  uint32_t push = 0, outInSmem = 0, outBytes = 0, chunkBytes = 0, queueCap = 0;  // push kernel (viterbi_fill_push.cu)
+  uint32_t C = 0, M = 0, threads = 0, tInSmem = 0, sPrevGlobal = 0, smemBytes = 0, nClusters = 0;
+  uint32_t outInSmem = 0, outBytes = 0, chunkBytes = 0, queueCap = 0;
   int32_t maxLen = -1;
 };
 
@@ -82,18 +83,16 @@ struct dnab_decoder {
   // user overrides
   uint32_t wantC = 0, wantThreads = 0, wantTMode = 0;  // tMode: 0 auto, 1 smem, 2 global
   uint32_t wantBlockMode = 0;   // transition table: 0 auto, 1 shared memory, 2 global memory
-  uint32_t idleSleepNs = 100;
   uint32_t tRecompute = 1;
   uint32_t thinN = 1024;  // push kernel, one-CTA machines: levels of at most this many states queue their successors directly (option "thin_n")
   uint32_t dealChunks = 8;  // push kernel, partition mode 3: DFS chunks dealt per CTA (option "deal_chunks")
   uint32_t queueCap = 0;    // push kernel: cap of the level queue, 0 = automatic (option "queue_cap")
   uint32_t wantSPrevMode = 0;   // S(pos-1): 0 auto, 1 shared memory, 2 global scratch
-  uint32_t wantKernel = 0;      // 0 push kernel (viterbi_fill_push.cu), 1 pull kernel (viterbi_kernels.cu)
   uint32_t wantPartition = 0;   // 0/1 index-order runs + in-degree sort (default), 2 DFS runs unsorted, 3 DFS chunks dealt round-robin + sort, 4 DFS runs + sort
   // device-resident structures for the current plan
   LaunchPlan plan;
   DevTables dev{};
-  DevBuf<uint32_t> dBlocks, dBlockOff, dSliceOff, dOrigId;
+  DevBuf<uint32_t> dBlocks, dBlockOff, dOrigId;
   DevBuf<uint32_t> dInChunks, dInChunkOff, dOutTable, dOutSliceOff, dOutOvf;
   DevBuf<uint4> dOutSlots;
   DevBuf<uint8_t> dSymChar;
@@ -114,7 +113,7 @@ struct dnab_decoder {
   DevBuf<long long> dFwdSweeps;
   bool debug = false;
   // read-batched kernel: 32 reads per group are the SIMD lanes (viterbi_fill_batch.cu)
-  int32_t wantBatch = -1;       // -1 auto (used when feasible and no push/pull tuning was requested), 0 off, 1 required
+  int32_t wantBatch = -1;       // -1 auto (used when feasible and no push-kernel tuning was requested), 0 off, 1 required
   uint32_t wantTeam = 0;        // CTAs per team (0 = smallest that fits)
   uint32_t wantWarps = 0;       // warps per CTA (0 = 32)
   BatchPlan bplan;
@@ -122,7 +121,7 @@ struct dnab_decoder {
                                 // transition that crosses CTAs; 32 = a 32nd of them, one class per lane of the polling warp)
   uint32_t eagerNotify = 0;     // option "eager_notify"
   uint32_t batchIdleNs = 100;   // option "batch_idle_ns"
-  uint32_t asyncClosure = 2;    // read-batched kernel: closure without level barriers: 0 off, 1 on, 2 automatic = in a team (option "async_closure")
+  uint32_t asyncClosure = 2;    // read-batched kernel: closure without level barriers: 0 off, 1 on, 2 automatic = on (option "async_closure")
   uint32_t teamSlackPct = 8;    // states per CTA above the balanced share that the partitioner may use (option "team_slack_pct")
   uint32_t wantPersist = 0;     // carried rows in the persisting part of L2 (option "persist_l2")
   size_t persistBytes = 0;
@@ -155,8 +154,8 @@ namespace dnab {
 
 // Alternative order of the states: depth-first preorder over the transition graph.  Cutting it
 // into C equal runs keeps more transitions inside one CTA (85% on the BASELINE config 2 machine
-// against 56% for index order) but measured slower on B200 (more closure sweeps per round), so
-// index order is the default and this is selectable (dnab_decoder_configure_ex).
+// against 56% for index order).  The push kernel deals chunks of it to the CTAs by default
+// (partition mode 3); option "partition" selects the others.
 static std::vector<uint32_t> dfsOrder(const dnab_decoder* d) {
   const uint32_t N = d->nStates;
   std::vector<uint32_t> outOff(N + 1, 0), outDst;
@@ -196,14 +195,12 @@ static std::vector<uint32_t> dfsOrder(const dnab_decoder* d) {
   return order;
 }
 
-// Word count of one CTA's slice of state blocks for cluster size C (used to decide whether
-// the slice fits in shared memory before the blocks are actually built).
+// Assignment of the states to the C CTAs of a cluster, and the state blocks of the traceback.
 struct Partition {
   uint32_t C = 0, M = 0;
   std::vector<uint32_t> newOf;   // reference state -> padded index g
   std::vector<uint32_t> origOf;  // padded index g -> reference state (0xFFFFFFFF = padding)
-  std::vector<uint32_t> blocks, blockOff, sliceOff;
-  uint32_t maxSliceWords = 0;
+  std::vector<uint32_t> blocks, blockOff;
 };
 
 static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
@@ -213,7 +210,7 @@ static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
   P.M = M;
   // 1. CTA assignment: equal runs of the reference's state order (default) or of a DFS order
   std::vector<uint32_t> order;
-  const uint32_t partMode = d->wantPartition ? d->wantPartition : (d->wantKernel == 0 ? 3u : 1u);
+  const uint32_t partMode = d->wantPartition ? d->wantPartition : 3u;
   const bool useDfs = partMode >= 2;
   if (C > 1 && useDfs)
     order = dfsOrder(d);
@@ -260,14 +257,8 @@ static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
   }
   P.blocks.clear();
   P.blockOff.assign(Np, 0);
-  P.sliceOff.assign(C + 1, 0);
-  P.maxSliceWords = 0;
   for (uint32_t g = 0; g < Np; ++g) {
     const uint32_t rank = g / M;
-    if (g % M == 0) {
-      while (P.blocks.size() % 8) P.blocks.push_back(0);  // slices start sector-aligned
-      P.sliceOff[rank] = (uint32_t)P.blocks.size();
-    }
     {
       // a block that fits one 32-byte sector must not straddle two (one L1/L2 access per state)
       const uint32_t s0 = P.origOf[g];
@@ -314,11 +305,7 @@ static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
       for (uint32_t dg : o) P.blocks.push_back((dg % M) | ((dg / M) << 20) | (dg / M != rank ? kEdgeRemote : 0u));
     }
     if (P.blocks.size() & 1) P.blocks.push_back(0);
-    if ((g + 1) % M == 0) P.sliceOff[rank + 1] = (uint32_t)P.blocks.size();
   }
-  // slice r ends where slice r+1 begins (after that slice's sector alignment): size the shared-memory
-  // copy from the final offsets
-  for (uint32_t r = 0; r < C; ++r) P.maxSliceWords = std::max(P.maxSliceWords, P.sliceOff[r + 1] - P.sliceOff[r]);
   return DNAB_OK;
 }
 
@@ -445,7 +432,12 @@ static uint32_t pushThreads(const dnab_decoder* d, uint32_t M) {
   return std::max<uint32_t>(32, std::min<uint32_t>(1024, (threads + 31) / 32 * 32));
 }
 
-static int buildPlanPush(dnab_decoder* d, int32_t planLen) {
+// Plan of the push kernel for reads of up to maxLen bases: cluster size, placements, tables, scratch.  The handle
+// keeps its current plan until the new one is complete; a failure after the first upload (which replaces buffers the
+// current plan points at) leaves no plan, so the next call builds one from scratch.
+static int buildPlan(dnab_decoder* d, int32_t maxLen) {
+  if (d->plan.maxLen >= maxLen && d->plan.C) return DNAB_OK;
+  const int32_t planLen = std::max(maxLen, 1024);
   const uint32_t N = d->nStates, k = d->k;
   LaunchPlan best;
   Partition P;
@@ -494,7 +486,6 @@ static int buildPlanPush(dnab_decoder* d, int32_t planLen) {
         best.chunkBytes = T.maxChunkBytes;
         best.queueCap = qCap;
         best.smemBytes = smem;
-        best.push = 1;
         break;
       }
     }
@@ -507,12 +498,46 @@ static int buildPlanPush(dnab_decoder* d, int32_t planLen) {
   }
   best.maxLen = planLen;
   const uint32_t C = best.C, M = best.M;
+
+  DevTables t{};
+  t.nStates = N;
+  t.M = M;
+  t.C = C;
+  t.k = k;
+  t.local = d->local;
+  t.nSyms = (uint32_t)d->symChar.size();
+  t.startG = P.newOf[0];
+  t.endG = P.newOf[N - 1];
+  t.tInSmem = best.tInSmem;
+  t.sPrevInSmem = best.sPrevGlobal ? 0 : 1;
+  t.outInSmem = best.outInSmem;
+  t.chunkStates = T.chunkStates;
+  t.nChunks = T.nChunks;
+  t.maxChunkBytes = T.maxChunkBytes;
+  t.maxOutBytes = T.maxOutBytes;
+  for (int i = 0; i < kMaxSyms; ++i) t.symScore[i] = i < (int)d->symScore.size() ? d->symScore[i] : 0.;
+  std::memcpy(t.sub, d->sub, sizeof t.sub);
+  std::memcpy(t.len, d->len, sizeof t.len);
+  t.noGap = d->noGap;
+  t.delOpen = d->delOpen;
+  t.delExtend = d->delExtend;
+  t.delEnd = d->delEnd;
+  t.tanDup = d->tanDup;
+  int nClusters = 0;
+  CUDA_TRY(queryMaxClustersPush(t, best.threads, best.smemBytes, &nClusters));
+  if (nClusters < 1) {
+    setLastError("no cluster of size " + std::to_string(C) + " can be resident on this device");
+    return DNAB_ECUDA;
+  }
+  best.nClusters = (uint32_t)nClusters;
+
+  // the uploads replace buffers the current plan points at: from here on a failure leaves no plan
+  d->plan = LaunchPlan();
   P.blocks.resize(P.blocks.size() + 8, 0);
   T.inChunks.resize(T.inChunks.size() + 4, 0);
   T.outTable.resize(T.outTable.size() + 4, 0);
-  CUDA_TRY(d->dBlocks.upload(P.blocks));  // the traceback kernel decodes records against the state blocks
+  CUDA_TRY(d->dBlocks.upload(P.blocks));
   CUDA_TRY(d->dBlockOff.upload(P.blockOff));
-  CUDA_TRY(d->dSliceOff.upload(P.sliceOff));
   CUDA_TRY(d->dOrigId.upload(P.origOf));
   CUDA_TRY(d->dSymChar.upload(d->symChar));
   CUDA_TRY(d->dInChunks.upload(T.inChunks));
@@ -521,29 +546,11 @@ static int buildPlanPush(dnab_decoder* d, int32_t planLen) {
   CUDA_TRY(d->dOutSliceOff.upload(T.outSliceOff));
   CUDA_TRY(d->dOutSlots.upload(T.outSlots));
   CUDA_TRY(d->dOutOvf.upload(T.outOvf));
-
-  DevTables& t = d->dev;
-  t = DevTables{};
-  t.nStates = N;
-  t.M = M;
-  t.C = C;
-  t.k = k;
-  t.local = d->local;
-  t.nSyms = (uint32_t)d->symChar.size();
-  t.startG = P.newOf[0];
-  t.endG = P.newOf[N - 1];
-  t.tInSmem = best.tInSmem;
-  t.blocksInSmem = 0;
-  t.sPrevGlobal = best.sPrevGlobal;
-  t.sPrevInSmem = best.sPrevGlobal ? 0 : 1;
-  t.outInSmem = best.outInSmem;
-  t.chunkStates = T.chunkStates;
-  t.nChunks = T.nChunks;
-  t.maxChunkBytes = T.maxChunkBytes;
-  t.maxOutBytes = T.maxOutBytes;
+  if (!best.tInSmem && k) CUDA_TRY(d->dTScratch.ensure((size_t)nClusters * C * k * M));
+  CUDA_TRY(d->dS0Scratch.ensure((size_t)nClusters * C * M));
+  if (best.sPrevGlobal) CUDA_TRY(d->dSScratch.ensure((size_t)nClusters * 2 * C * M));
   t.blocks = d->dBlocks.p;
   t.blockOff = d->dBlockOff.p;
-  t.sliceOff = d->dSliceOff.p;
   t.origId = d->dOrigId.p;
   t.symChar = d->dSymChar.p;
   t.inChunks = d->dInChunks.p;
@@ -552,131 +559,7 @@ static int buildPlanPush(dnab_decoder* d, int32_t planLen) {
   t.outSliceOff = d->dOutSliceOff.p;
   t.outSlots = d->dOutSlots.p;
   t.outOvf = d->dOutOvf.p;
-  for (int i = 0; i < kMaxSyms; ++i) t.symScore[i] = i < (int)d->symScore.size() ? d->symScore[i] : 0.;
-  std::memcpy(t.sub, d->sub, sizeof t.sub);
-  std::memcpy(t.len, d->len, sizeof t.len);
-  t.noGap = d->noGap;
-  t.delOpen = d->delOpen;
-  t.delExtend = d->delExtend;
-  t.delEnd = d->delEnd;
-  t.tanDup = d->tanDup;
-
-  int nClusters = 0;
-  CUDA_TRY(queryMaxClustersPush(t, best.threads, best.smemBytes, &nClusters));
-  if (nClusters < 1) {
-    setLastError("no cluster of size " + std::to_string(C) + " can be resident on this device");
-    return DNAB_ECUDA;
-  }
-  best.nClusters = (uint32_t)nClusters;
-  if (!best.tInSmem && k) CUDA_TRY(d->dTScratch.ensure((size_t)nClusters * C * k * M));
-  CUDA_TRY(d->dS0Scratch.ensure((size_t)nClusters * C * M));
-  if (best.sPrevGlobal) CUDA_TRY(d->dSScratch.ensure((size_t)nClusters * 2 * C * M));
-  d->plan = best;
-  return DNAB_OK;
-}
-
-static int buildPlan(dnab_decoder* d, int32_t maxLen) {
-  if (d->plan.maxLen >= maxLen && d->plan.C) return DNAB_OK;
-  const uint32_t N = d->nStates, k = d->k;
-  const int32_t planLen = std::max(maxLen, 1024);
-  if (d->wantKernel == 0) return buildPlanPush(d, planLen);
-  // Preference: the smallest cluster that holds the three live columns; within it, keep the T
-  // columns and the CTA's slice of the transition table in shared memory when they fit too.
-  LaunchPlan best;
-  Partition P;
-  // more reads in flight beats more SMs per read (measured), so the smallest feasible cluster wins;
-  // any size up to 16 is allowed, not only powers of two
-  std::vector<uint32_t> cands = {1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 14, 16};
-  if (d->wantC >= 1 && d->wantC <= (uint32_t)kMaxCluster) cands = {d->wantC};  // any size, not only powers of two
-  for (uint32_t C : cands) {
-    const uint32_t M = (N + C - 1) / C;
-    if (M > 65535) continue;  // 16-bit local indices in the out-edge words
-    if (makeLayout(M, k, 0, 0, (uint32_t)planLen, d->wantSPrevMode == 1 ? 0 : 1).total > d->smemOptin) continue;
-    int rc = buildPartition(d, C, P);
-    if (rc != DNAB_OK) return rc;
-    // options in order of preference: S(pos-1) in shared memory before global scratch; within that
-    // (T,blocks) in smem, blocks only, T only, neither
-    const uint32_t opts[4][2] = {{1, 1}, {0, 1}, {1, 0}, {0, 0}};
-    for (uint32_t sg = 0; sg < 2 && !best.C; ++sg) {
-      if (d->wantSPrevMode == 1 && sg) continue;
-      if (d->wantSPrevMode == 2 && !sg) continue;
-      for (const auto& o : opts) {
-        const uint32_t tIn = (k == 0) ? 0 : o[0], bIn = o[1];
-        if (d->wantTMode == 1 && k && !tIn) continue;
-        if (d->wantTMode == 2 && tIn) continue;
-        if (d->wantBlockMode == 1 && !bIn) continue;
-        if (d->wantBlockMode == 2 && bIn) continue;
-        const uint32_t smem = makeLayout(M, k, tIn, bIn ? P.maxSliceWords : 0, (uint32_t)planLen, sg).total;
-        if (smem <= d->smemOptin) {
-          best.C = C;
-          best.M = M;
-          best.tInSmem = tIn;
-          best.blocksInSmem = bIn;
-          best.sPrevGlobal = sg;
-          best.smemBytes = smem;
-          break;
-        }
-      }
-    }
-    if (best.C) break;
-  }
-  if (!best.C) {
-    setLastError("machine does not fit: " + std::to_string(N) +
-                 " states need more shared memory than a 16-CTA cluster has (or the requested configuration is infeasible)");
-    return DNAB_EINVAL;
-  }
-  // small slices: few threads per CTA so that several CTAs (reads) share an SM; large slices: more warps
-  // to overlap the latency-bound per-state chains (measured on B200)
-  uint32_t threads = d->wantThreads ? d->wantThreads
-                     : best.M <= 1024 ? 128 : best.M <= 2048 ? 256 : best.M <= 6000 ? 512 : 768;
-  threads = std::min<uint32_t>(1024, (threads + 31) / 32 * 32);
-  best.threads = threads;
-  best.maxLen = planLen;
-  best.sliceWords = P.maxSliceWords;
-
-  const uint32_t C = best.C, M = best.M;
-  P.blocks.resize(P.blocks.size() + 8, 0);
-  CUDA_TRY(d->dBlocks.upload(P.blocks));
-  CUDA_TRY(d->dBlockOff.upload(P.blockOff));
-  CUDA_TRY(d->dSliceOff.upload(P.sliceOff));
-  CUDA_TRY(d->dOrigId.upload(P.origOf));
-  CUDA_TRY(d->dSymChar.upload(d->symChar));
-
-  DevTables& t = d->dev;
-  t.nStates = N;
-  t.M = M;
-  t.C = C;
-  t.k = k;
-  t.local = d->local;
-  t.nSyms = (uint32_t)d->symChar.size();
-  t.startG = P.newOf[0];
-  t.endG = P.newOf[N - 1];
-  t.tInSmem = best.tInSmem;
-  t.blocksInSmem = best.blocksInSmem;
-  t.sPrevGlobal = best.sPrevGlobal;
-  t.blocks = d->dBlocks.p;
-  t.blockOff = d->dBlockOff.p;
-  t.sliceOff = d->dSliceOff.p;
-  t.origId = d->dOrigId.p;
-  t.symChar = d->dSymChar.p;
-  for (int i = 0; i < kMaxSyms; ++i) t.symScore[i] = i < (int)d->symScore.size() ? d->symScore[i] : 0.;
-  std::memcpy(t.sub, d->sub, sizeof t.sub);
-  std::memcpy(t.len, d->len, sizeof t.len);
-  t.noGap = d->noGap;
-  t.delOpen = d->delOpen;
-  t.delExtend = d->delExtend;
-  t.delEnd = d->delEnd;
-  t.tanDup = d->tanDup;
-
-  int nClusters = 0;
-  CUDA_TRY(queryMaxClusters(t, best.threads, best.smemBytes, &nClusters));
-  if (nClusters < 1) {
-    setLastError("no cluster of size " + std::to_string(C) + " can be resident on this device");
-    return DNAB_ECUDA;
-  }
-  best.nClusters = (uint32_t)nClusters;
-  if (!best.tInSmem && k) CUDA_TRY(d->dTScratch.ensure((size_t)nClusters * C * k * M));
-  if (best.sPrevGlobal) CUDA_TRY(d->dSScratch.ensure((size_t)nClusters * 2 * C * M));
+  d->dev = t;
   d->plan = best;
   return DNAB_OK;
 }
@@ -781,19 +664,20 @@ static std::vector<uint32_t> growPartition(const dnab_decoder* d, uint32_t T, ui
 static bool batchWanted(const dnab_decoder* d) {
   if (d->wantBatch == 0) return false;
   if (d->wantBatch == 1) return true;
-  // automatic: the batched kernel, unless the caller tuned the one-read-per-cluster kernels explicitly
-  return !(d->wantC || d->wantThreads || d->wantTMode || d->wantBlockMode || d->wantSPrevMode || d->wantKernel ||
-           d->wantPartition);
+  // automatic: the batched kernel, unless the caller tuned the one-read-per-cluster push kernel explicitly
+  return !(d->wantC || d->wantThreads || d->wantTMode || d->wantBlockMode || d->wantSPrevMode || d->wantPartition);
 }
 
+// Plan of the read-batched kernel.  It depends on the options only, so the answer "infeasible" is kept until an option
+// changes.  The plan is built in locals and committed at the end; a failure after the first upload leaves no plan.
 static int buildBatchPlan(dnab_decoder* d) {
-  BatchPlan& bp = d->bplan;
-  if (bp.ready) {
-    if (!bp.feasible) setLastError("the read-batched kernel cannot take this machine");
-    return bp.feasible ? DNAB_OK : DNAB_EINVAL;
+  if (d->bplan.ready) {
+    if (!d->bplan.feasible) setLastError("the read-batched kernel cannot take this machine");
+    return d->bplan.feasible ? DNAB_OK : DNAB_EINVAL;
   }
-  bp.ready = true;
-  bp.feasible = false;
+  d->bplan.ready = true;  // infeasible until committed below
+  BatchPlan bp;
+  BatchTables t{};
   const uint32_t N = d->nStates, k = d->k;
   // warps per CTA (measured on B200): 24 when one CTA holds the group (80 registers, no spills: 349k vs 315k reads/s on
   // dnastore-l4), 32 in a team (more states relaxed side by side per level: 1,120 vs 1,060 reads/s on the 46,670-state machine)
@@ -972,7 +856,6 @@ static int buildBatchPlan(dnab_decoder* d) {
     bp.warps = W;
     bp.smemBytes = smem;
     bp.crossFraction = total ? (double)cross / (double)total : 0.;
-    BatchTables& t = d->btab;
     t = BatchTables{};
     t.nStates = N;
     t.M = M;
@@ -1020,40 +903,6 @@ static int buildBatchPlan(dnab_decoder* d) {
                  " states x 32 reads x 16 bytes exceed the shared memory of " + std::to_string(maxTeam) + " SMs");
     return DNAB_EINVAL;
   }
-  BatchTables& t = d->btab;
-  inE.push_back(make_uint2(0, 0));
-  outE.push_back(0);
-  CUDA_TRY(d->dbHdr.upload(hdr));
-  CUDA_TRY(d->dbIn.upload(inE));
-  relE.push_back(make_uint2(0, 0));
-  CUDA_TRY(d->dbRel.upload(relE));
-  CUDA_TRY(d->dbHdr2.upload(hdr2));
-  CUDA_TRY(d->dbOut.upload(outE));
-  CUDA_TRY(d->dbRankInOff.upload(rankInOff));
-  CUDA_TRY(d->dbRankOutOff.upload(rankOutOff));
-  CUDA_TRY(d->dbRemoteIn.upload(remoteIn));
-  CUDA_TRY(d->dbClsOff.upload(clsOff));
-  CUDA_TRY(d->dbClsStates.upload(clsStates));
-  // score tables with the traceback's association, formed once on the host in IEEE fp64 (-ffp-contract=off)
-  std::vector<double> tsE((size_t)kMaxSyms * 16, 0.);
-  for (uint32_t sym = 0; sym < d->symScore.size(); ++sym)
-    for (uint32_t b = 0; b < 4; ++b)
-      for (uint32_t x = 0; x < 4; ++x) {
-        volatile double a = d->symScore[sym] + d->noGap;  // (score + noGap) + sub, src/viterbi.cpp:255
-        tsE[(sym * 4 + b) * 4 + x] = a + d->sub[b * 4 + x];
-      }
-  CUDA_TRY(d->dbTsE.upload(tsE));
-  t.hdr = d->dbHdr.p;
-  t.inEdges = d->dbIn.p;
-  t.outEdges = d->dbOut.p;
-  t.rankInOff = d->dbRankInOff.p;
-  t.rankOutOff = d->dbRankOutOff.p;
-  t.remoteIn = d->dbRemoteIn.p;
-  t.clsOff = d->dbClsOff.p;
-  t.clsStates = d->dbClsStates.p;
-  t.hdr2 = d->dbHdr2.p;
-  t.relEdges = d->dbRel.p;
-  t.tsE = d->dbTsE.p;
   for (int i = 0; i < kMaxSyms; ++i) {
     const double sc = i < (int)d->symScore.size() ? d->symScore[i] : 0.;
     t.symScore[i] = sc;
@@ -1070,6 +919,43 @@ static int buildBatchPlan(dnab_decoder* d) {
   t.delExtend = d->delExtend;
   t.delEnd = d->delEnd;
   t.tanDup = d->tanDup;
+  int perSm = 0;
+  CUDA_TRY(queryBatchTeams(t, bp.warps, bp.smemBytes, &perSm));
+  if (perSm < 1) {
+    setLastError("the read-batched kernel does not fit an SM");
+    return DNAB_ECUDA;
+  }
+  bp.ctasPerSm = (uint32_t)perSm;
+  bp.nTeams = (uint32_t)d->smCount * bp.ctasPerSm / bp.T;
+  if (bp.nTeams < 1) {
+    setLastError("a team of " + std::to_string(bp.T) + " CTAs cannot be resident at once");
+    return DNAB_EINVAL;
+  }
+
+  // a failure from here on says nothing about the machine: it leaves no plan, and the next call tries again
+  d->bplan = BatchPlan();
+  inE.push_back(make_uint2(0, 0));
+  outE.push_back(0);
+  relE.push_back(make_uint2(0, 0));
+  // score tables with the traceback's association, formed once on the host in IEEE fp64 (-ffp-contract=off)
+  std::vector<double> tsE((size_t)kMaxSyms * 16, 0.);
+  for (uint32_t sym = 0; sym < d->symScore.size(); ++sym)
+    for (uint32_t b = 0; b < 4; ++b)
+      for (uint32_t x = 0; x < 4; ++x) {
+        volatile double a = d->symScore[sym] + d->noGap;  // (score + noGap) + sub, src/viterbi.cpp:255
+        tsE[(sym * 4 + b) * 4 + x] = a + d->sub[b * 4 + x];
+      }
+  CUDA_TRY(d->dbHdr.upload(hdr));
+  CUDA_TRY(d->dbIn.upload(inE));
+  CUDA_TRY(d->dbRel.upload(relE));
+  CUDA_TRY(d->dbHdr2.upload(hdr2));
+  CUDA_TRY(d->dbOut.upload(outE));
+  CUDA_TRY(d->dbRankInOff.upload(rankInOff));
+  CUDA_TRY(d->dbRankOutOff.upload(rankOutOff));
+  CUDA_TRY(d->dbRemoteIn.upload(remoteIn));
+  CUDA_TRY(d->dbClsOff.upload(clsOff));
+  CUDA_TRY(d->dbClsStates.upload(clsStates));
+  CUDA_TRY(d->dbTsE.upload(tsE));
   // traceback tables in reference order
   CUDA_TRY(d->dbEmitOff.upload(d->emitOff));
   CUDA_TRY(d->dbEmitSrc.upload(d->emitSrc));
@@ -1078,32 +964,6 @@ static int buildBatchPlan(dnab_decoder* d) {
   CUDA_TRY(d->dbNullSrc.upload(d->nullSrc));
   CUDA_TRY(d->dbNullSym.upload(d->nullSym));
   CUDA_TRY(d->dSymChar.upload(d->symChar));
-  BatchTraceTables& tt = d->btrace;
-  tt.nStates = N;
-  tt.k = k;
-  tt.local = d->local;
-  tt.T = bp.T * bp.warps;
-  tt.emitOff = d->dbEmitOff.p;
-  tt.emitSrc = d->dbEmitSrc.p;
-  tt.emitSym = d->dbEmitSym.p;
-  tt.nullOff = d->dbNullOff.p;
-  tt.nullSrc = d->dbNullSrc.p;
-  tt.nullSym = d->dbNullSym.p;
-  tt.symChar = d->dSymChar.p;
-  int perSm = 0;
-  CUDA_TRY(queryBatchTeams(t, bp.warps, bp.smemBytes, &perSm));
-  if (perSm < 1) {
-    bp.feasible = false;
-    setLastError("the read-batched kernel does not fit an SM");
-    return DNAB_ECUDA;
-  }
-  bp.ctasPerSm = (uint32_t)perSm;
-  bp.nTeams = (uint32_t)d->smCount * bp.ctasPerSm / bp.T;
-  if (bp.nTeams < 1) {
-    bp.feasible = false;
-    setLastError("a team of " + std::to_string(bp.T) + " CTAs cannot be resident at once");
-    return DNAB_EINVAL;
-  }
   const size_t Np = (size_t)bp.T * bp.M;
   CUDA_TRY(d->dbPriv.ensure((size_t)bp.nTeams * Np * (2 + k) * 32));
   {
@@ -1123,7 +983,55 @@ static int buildBatchPlan(dnab_decoder* d) {
   CUDA_TRY(d->dbTeamState.ensure((size_t)bp.nTeams * bp.T * kNotifyClasses));
   CUDA_TRY(d->dbTeamPassive.ensure((size_t)bp.nTeams * 2));
   CUDA_TRY(d->dbBarrier.ensure((size_t)bp.nTeams));
+  t.hdr = d->dbHdr.p;
+  t.inEdges = d->dbIn.p;
+  t.outEdges = d->dbOut.p;
+  t.rankInOff = d->dbRankInOff.p;
+  t.rankOutOff = d->dbRankOutOff.p;
+  t.remoteIn = d->dbRemoteIn.p;
+  t.clsOff = d->dbClsOff.p;
+  t.clsStates = d->dbClsStates.p;
+  t.hdr2 = d->dbHdr2.p;
+  t.relEdges = d->dbRel.p;
+  t.tsE = d->dbTsE.p;
+  BatchTraceTables tt{};
+  tt.nStates = N;
+  tt.k = k;
+  tt.local = d->local;
+  tt.T = bp.T * bp.warps;
+  tt.emitOff = d->dbEmitOff.p;
+  tt.emitSrc = d->dbEmitSrc.p;
+  tt.emitSym = d->dbEmitSym.p;
+  tt.nullOff = d->dbNullOff.p;
+  tt.nullSrc = d->dbNullSrc.p;
+  tt.nullSym = d->dbNullSym.p;
+  tt.symChar = d->dSymChar.p;
+  d->btab = t;
+  d->btrace = tt;
+  bp.ready = true;
+  d->bplan = bp;
   return DNAB_OK;
+}
+
+// The (start, mid, end) events of one fill + traceback launch pair: the handle's own triple when the caller times the
+// call itself (host-buffer path), a triple from the pool when device-path timing is on (resolved in get_stats).
+static cudaError_t takeEvents(dnab_decoder* d, bool timeIt, cudaEvent_t ev[3], bool* rec) {
+  ev[0] = d->ev0;
+  ev[1] = d->ev1;
+  ev[2] = d->ev2;
+  const bool pooled = d->timing && !timeIt;
+  if (pooled) {
+    while (d->evPool.size() < d->evUsed + 3) {
+      cudaEvent_t e;
+      const cudaError_t err = cudaEventCreate(&e);
+      if (err != cudaSuccess) return err;
+      d->evPool.push_back(e);
+    }
+    for (int i = 0; i < 3; ++i) ev[i] = d->evPool[d->evUsed + i];
+    d->evUsed += 3;
+  }
+  *rec = timeIt || pooled;
+  return cudaSuccess;
 }
 
 // fill + traceback with the read-batched kernel; hostLen (optional) lets the groups be formed from reads of similar length
@@ -1161,8 +1069,7 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
     a.nGroups = n;
     a.nTeams = (uint32_t)std::min<int64_t>(bp.nTeams, n);
     a.maxLen = maxLen;
-    // measured on B200: without level barriers a team gains 10-60 % (1,250 vs 1,130 reads/s on the 46,670-state machine, 5.9k vs
-    // 3.6k on watermark64.1*l4); a single CTA loses 5 % (331k vs 349k reads/s on dnastore-l4: its levels are short and dense)
+    // automatic (2) = no level barriers, in a team and in a single CTA alike; the numbers of DESIGN.md 6 were measured so
     a.asyncClosure = d->asyncClosure == 2 ? 1u : d->asyncClosure;
     a.idleNs = d->batchIdleNs;
     a.packed = dPacked;
@@ -1181,28 +1088,17 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
     a.partOrig = d->dbPartOrig.p;
     a.cells = at == 0 ? dCells : nullptr;
     a.dbg = d->debug ? d->dDbg.p : nullptr;
-    cudaEvent_t e0 = d->ev0, e1 = d->ev1, e2 = d->ev2;
-    const bool pooled = d->timing && !timeIt;
-    if (pooled) {
-      while (d->evPool.size() < d->evUsed + 3) {
-        cudaEvent_t e;
-        CUDA_TRY(cudaEventCreate(&e));
-        d->evPool.push_back(e);
-      }
-      e0 = d->evPool[d->evUsed];
-      e1 = d->evPool[d->evUsed + 1];
-      e2 = d->evPool[d->evUsed + 2];
-      d->evUsed += 3;
-    }
-    const bool rec = timeIt || pooled;
+    cudaEvent_t ev[3];
+    bool rec = false;
+    CUDA_TRY(takeEvents(d, timeIt, ev, &rec));
     if (bp.T > 1) {
       CUDA_TRY(cudaMemsetAsync(d->dbTeamState.p, 0, d->dbTeamState.n * sizeof(uint32_t), stream));
       CUDA_TRY(cudaMemsetAsync(d->dbTeamPassive.p, 0, d->dbTeamPassive.n * sizeof(uint32_t), stream));
       CUDA_TRY(cudaMemsetAsync(d->dbBarrier.p, 0, d->dbBarrier.n * sizeof(unsigned long long), stream));
     }
-    if (rec) CUDA_TRY(cudaEventRecord(e0, stream));
+    if (rec) CUDA_TRY(cudaEventRecord(ev[0], stream));
     CUDA_TRY(launchFillBatch(d->btab, a, bp.warps, bp.smemBytes, stream, d->persistBytes));
-    if (rec) CUDA_TRY(cudaEventRecord(e1, stream));
+    if (rec) CUDA_TRY(cudaEventRecord(ev[1], stream));
     BatchTraceArgs ta{};
     ta.nSlots = n * 32;
     ta.maxLen = maxLen;
@@ -1222,7 +1118,7 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
     ta.pathStride = pathStride;
     ta.pathLen = dPathLen;
     CUDA_TRY(launchTracebackBatch(d->btrace, ta, stream));
-    if (rec) CUDA_TRY(cudaEventRecord(e2, stream));
+    if (rec) CUDA_TRY(cudaEventRecord(ev[2], stream));
     d->stats.kernel_launches += 2;
     d->stats.fill_launches += 1;
     d->stats.traceback_launches += 1;
@@ -1272,14 +1168,9 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
   for (int64_t at = 0; at < nReads; at += chunk) {
     const int64_t n = std::min(chunk, nReads - at);
     FillArgs fa{};
-    if (d->plan.push)
-      fa.play = makePushLayout(d->plan.M, d->k, d->plan.tInSmem, d->plan.sPrevGlobal ? 0 : 1, d->plan.outBytes,
-                               d->plan.chunkBytes, d->dev.nChunks, (uint32_t)d->plan.maxLen, d->plan.queueCap);
-    else
-      fa.lay = makeLayout(d->plan.M, d->k, d->plan.tInSmem, d->plan.blocksInSmem ? d->plan.sliceWords : 0,
-                          (uint32_t)d->plan.maxLen, d->plan.sPrevGlobal);
+    fa.play = makePushLayout(d->plan.M, d->k, d->plan.tInSmem, d->plan.sPrevGlobal ? 0 : 1, d->plan.outBytes,
+                             d->plan.chunkBytes, d->dev.nChunks, (uint32_t)d->plan.maxLen, d->plan.queueCap);
     fa.nReads = n;
-    fa.idleSleepNs = d->idleSleepNs;
     fa.thinN = d->thinN;
     fa.tRecompute = d->tRecompute;
     fa.maxLen = maxLen;
@@ -1298,31 +1189,15 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
     fa.cells = at == 0 ? dCells : nullptr;
     fa.dbg = d->debug ? d->dDbg.p : nullptr;
     const uint32_t nClusters = (uint32_t)std::min<int64_t>(d->plan.nClusters, n);
-    cudaEvent_t e0 = d->ev0, e1 = d->ev1, e2 = d->ev2;
-    const bool pooled = d->timing && !timeIt;
-    if (pooled) {
-      while (d->evPool.size() < d->evUsed + 3) {
-        cudaEvent_t e;
-        CUDA_TRY(cudaEventCreate(&e));
-        d->evPool.push_back(e);
-      }
-      e0 = d->evPool[d->evUsed];
-      e1 = d->evPool[d->evUsed + 1];
-      e2 = d->evPool[d->evUsed + 2];
-      d->evUsed += 3;
-    }
-    const bool rec = timeIt || pooled;
-    if (rec) CUDA_TRY(cudaEventRecord(e0, stream));
-    if (d->plan.push) {
-      CUDA_TRY(d->dNextRead.ensure(1));
-      CUDA_TRY(cudaMemsetAsync(d->dNextRead.p, 0, sizeof(unsigned long long), stream));
-      fa.nextRead = d->dNextRead.p;
-    }
-    if (d->plan.push)
-      CUDA_TRY(launchFillPush(d->dev, fa, nClusters, d->plan.threads, d->plan.smemBytes, stream));
-    else
-      CUDA_TRY(launchFill(d->dev, fa, nClusters, d->plan.threads, d->plan.smemBytes, stream));
-    if (rec) CUDA_TRY(cudaEventRecord(e1, stream));
+    cudaEvent_t ev[3];
+    bool rec = false;
+    CUDA_TRY(takeEvents(d, timeIt, ev, &rec));
+    if (rec) CUDA_TRY(cudaEventRecord(ev[0], stream));
+    CUDA_TRY(d->dNextRead.ensure(1));
+    CUDA_TRY(cudaMemsetAsync(d->dNextRead.p, 0, sizeof(unsigned long long), stream));
+    fa.nextRead = d->dNextRead.p;
+    CUDA_TRY(launchFillPush(d->dev, fa, nClusters, d->plan.threads, d->plan.smemBytes, stream));
+    if (rec) CUDA_TRY(cudaEventRecord(ev[1], stream));
     TracebackArgs ta{};
     ta.nReads = n;
     ta.maxLen = maxLen;
@@ -1341,7 +1216,7 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
     ta.pathStride = pathStride;
     ta.pathLen = dPathLen ? dPathLen + at : nullptr;
     CUDA_TRY(launchTraceback(d->dev, ta, stream));
-    if (rec) CUDA_TRY(cudaEventRecord(e2, stream));
+    if (rec) CUDA_TRY(cudaEventRecord(ev[2], stream));
     d->stats.kernel_launches += 2;
     d->stats.fill_launches += 1;
     d->stats.traceback_launches += 1;
@@ -1473,17 +1348,6 @@ int dnab_decoder_configure(dnab_decoder* d, uint32_t cluster_size, uint32_t thre
   return DNAB_OK;
 }
 
-int dnab_decoder_configure_ex(dnab_decoder* d, uint32_t block_table_mode, uint32_t partition_mode) {
-  if (!d) return DNAB_EINVAL;
-  // kept for round-1 callers: decimal digits select two things each; new code uses dnab_decoder_set_option
-  d->wantBlockMode = block_table_mode % 10;
-  d->wantSPrevMode = block_table_mode / 10;
-  d->wantPartition = partition_mode % 10;
-  d->wantKernel = partition_mode / 10;
-  d->plan = LaunchPlan();
-  return DNAB_OK;
-}
-
 int dnab_decoder_set_option(dnab_decoder* d, const char* key, int64_t value) {
   if (!d || !key || value < 0) {
     setLastError("dnab_decoder_set_option: bad argument");
@@ -1491,13 +1355,13 @@ int dnab_decoder_set_option(dnab_decoder* d, const char* key, int64_t value) {
   }
   const std::string k(key);
   const uint32_t v = (uint32_t)value;
-  if (k == "kernel") {  // 0 automatic, 1 read-batched, 2 push (one read per cluster), 3 pull
-    if (v > 3) {
-      setLastError("dnab_decoder_set_option: kernel must be 0..3");
+  if (k == "kernel") {  // 0 automatic, 1 read-batched, 2 push (one read per cluster)
+    if (v > 2) {
+      setLastError(v == 3 ? "dnab_decoder_set_option: kernel 3 (the pull-closure fill kernel) was retired; use 0, 1 or 2"
+                          : "dnab_decoder_set_option: kernel must be 0, 1 or 2");
       return DNAB_EINVAL;
     }
     d->wantBatch = v == 0 ? -1 : v == 1 ? 1 : 0;
-    d->wantKernel = v == 3 ? 1 : 0;
   } else if (k == "team_size")
     d->wantTeam = v;
   else if (k == "warps_per_cta")
@@ -1522,9 +1386,9 @@ int dnab_decoder_set_option(dnab_decoder* d, const char* key, int64_t value) {
     d->queueCap = v;
   else if (k == "deal_chunks")
     d->dealChunks = v;
-  else if (k == "idle_sleep_ns")
-    d->idleSleepNs = v;
-  else if (k == "eager_notify")
+  else if (k == "idle_sleep_ns") {
+    // back-off of the retired pull-closure kernel: still accepted so that existing callers keep working; no effect
+  } else if (k == "eager_notify")
     d->eagerNotify = v;
   else if (k == "notify_classes")
     d->notifyClasses = v;
@@ -1579,7 +1443,7 @@ int dnab_decoder_get_info(const dnab_decoder* dc, dnab_decoder_info* info) {
   info->threads_per_cta = d->plan.threads;
   info->smem_bytes_per_cta = d->plan.smemBytes;
   info->t_in_smem = d->plan.tInSmem;
-  info->table_in_smem = d->plan.push ? d->plan.outInSmem : d->plan.blocksInSmem;
+  info->table_in_smem = d->plan.outInSmem;
   info->s_prev_in_smem = d->plan.sPrevGlobal ? 0 : 1;
   info->n_clusters = d->plan.nClusters;
   info->sm_count = (uint32_t)d->smCount;

@@ -1,5 +1,5 @@
-// Device-side table layout shared by the kernels (viterbi_kernels.cu) and the
-// host code that builds it (decoder.cu).
+// Device-side table layout of the one-read-per-cluster Viterbi path, shared by its kernels
+// (viterbi_fill_push.cu, viterbi_traceback.cu) and the host code that builds it (decoder.cu).
 #pragma once
 #include <cstdint>
 
@@ -11,9 +11,10 @@ constexpr int kMaxCluster = 16;
 constexpr uint32_t kNoPred = 255;  // predecessor record: "no candidate"
 
 // ---------------------------------------------------------------------------
-// State blocks.  The padded state space (Np = C*M states; state g lives in CTA
-// rank g/M at local index g%M) is described by one block of 32-bit words per state,
-// 8-byte aligned, found through blockOff[g]:
+// State blocks: the traceback kernel decodes a predecessor record of state g against g's
+// block (the record is an index into g's incoming edges).  The padded state space (Np = C*M
+// states; state g lives in CTA rank g/M at local index g%M) is described by one block of
+// 32-bit words per state, 8-byte aligned, found through blockOff[g]:
 //
 //   word 0   nEmit | nIn<<8 | nOut<<16 | mdl<<24        (nIn = nEmit + nNull)
 //   word 1   ctx: 2 bits per duplication index i = tanDupBase(ss,i)
@@ -28,24 +29,18 @@ constexpr uint32_t kNoPred = 255;  // predecessor record: "no candidate"
 //   then     nOut outgoing edges, one word each (states to wake when this one grows):
 //              bits 0..15 local index, bits 20..23 rank, bit 24 "other CTA"
 //   padding to an even number of words.
-// Everything the inner loops need is pre-shifted so that an edge costs two ANDs.
+// Of these the traceback reads nEmit, nIn and the source and symbol of an incoming edge.
 // ---------------------------------------------------------------------------
 constexpr uint32_t kEdgeRemote = 1u << 24;
 __host__ __device__ inline uint32_t hdrNEmit(uint32_t w0) { return w0 & 0xFFu; }
 __host__ __device__ inline uint32_t hdrNIn(uint32_t w0) { return (w0 >> 8) & 0xFFu; }
-__host__ __device__ inline uint32_t hdrNOut(uint32_t w0) { return (w0 >> 16) & 0xFFu; }
-__host__ __device__ inline uint32_t hdrMdl(uint32_t w0) { return (w0 >> 24) & 0xFu; }
-__host__ __device__ inline uint32_t hdrCtx(uint32_t w1, uint32_t i) { return (w1 >> (2 * i)) & 0x3u; }
 __host__ __device__ inline uint32_t edgeOff(uint32_t a) { return a & 0xFFFFFu; }
 __host__ __device__ inline uint32_t edgeRank(uint32_t a) { return (a >> 20) & 0xFu; }
 __host__ __device__ inline uint32_t edgeSymOff(uint32_t b) { return b & 0xFFu; }
-__host__ __device__ inline uint32_t edgeTsEOff(uint32_t b) { return (b >> 8) & 0x1FFFu; }
-__host__ __device__ inline uint32_t edgeSubOff(uint32_t b) { return (b >> 8) & 0x60u; }  // base*32
-__host__ __device__ inline uint32_t outLocal(uint32_t w) { return w & 0xFFFFu; }
 
 // ---------------------------------------------------------------------------
 // Tables of the push kernel (viterbi_fill_push.cu).  Same padded state space and the same
-// partition as above; two compact forms of the transition table:
+// partition as the state blocks; two compact forms of the transition table:
 //
 //  * IN-TABLE, streamed.  The dense passes (emission, first closure pass, predecessor
 //    pass) visit the states of a CTA in index order, one state per thread and `chunkStates`
@@ -89,14 +84,10 @@ struct DevTables {
   uint32_t startG;    // padded-space index of reference state 0
   uint32_t endG;      // padded-space index of the reference's last state
   uint32_t tInSmem;   // T columns in shared memory (else in global scratch)
-  uint32_t blocksInSmem;  // every CTA keeps its slice of the state blocks in shared memory
-  uint32_t sPrevGlobal;   // the previous column S(pos-1) lives in global scratch (L2) instead of shared memory
-  const uint32_t* blocks;     // state blocks; the blocks of one CTA's slice are contiguous
+  const uint32_t* blocks;     // state blocks (traceback)
   const uint32_t* blockOff;   // [Np] word offset of each state's block
-  const uint32_t* sliceOff;   // [C+1] word offset where each rank's slice of `blocks` begins
   const uint32_t* origId;     // [Np] reference state index, 0xFFFFFFFF for padding
   const uint8_t* symChar;     // [nSyms] input-symbol character of each id
-  // push kernel
   uint32_t sPrevInSmem;       // S(pos-1) kept in shared memory (else in global scratch / L2)
   uint32_t outInSmem;         // the CTA's out-table is resident in shared memory
   uint32_t chunkStates;       // states per in-table chunk (= threads per CTA)

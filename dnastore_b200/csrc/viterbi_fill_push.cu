@@ -1,8 +1,8 @@
 // viterbiFillPushKernel: the ViterbiMatrix fill (reference src/viterbi.cpp:62-176) for a batch of
 // reads, one thread-block cluster per read, with the within-column closure done PUSH style.
 //
-// Why a second fill kernel.  The first one (viterbi_kernels.cu) relaxes dirty states PULL style: a hop
-// of a propagation chain costs two transition-table accesses (the state's incoming list, then its
+// Why push.  The project's first fill kernel (round 1, since retired) relaxed dirty states PULL style: a hop
+// of a propagation chain cost two transition-table accesses (the state's incoming list, then its
 // outgoing list to wake successors) that miss L1 (cluster barriers flush it), plus a bitmap /
 // compaction / pending-counter protocol: ~3,000 cycles per hop measured on B200, and a column of the
 // BASELINE config-2 machine has chains of 17-46 hops.  Here
@@ -28,7 +28,7 @@
 //     themselves, which saves the scan and one of the two CTA barriers of a level.
 // Everything else -- the emission step, the predecessor records evaluated with the TRACEBACK's own
 // floating-point association and candidate order (src/viterbi.cpp:251-286), duplication opens, the
-// record layout read by viterbiTracebackKernel -- is as in viterbi_kernels.cu.
+// record layout read by viterbiTracebackKernel (viterbi_traceback.cu) -- follows the reference directly.
 #include <cooperative_groups.h>
 #include <cuda_runtime.h>
 

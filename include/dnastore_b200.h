@@ -111,32 +111,32 @@ typedef struct dnab_decoder_info {
   uint32_t threads_per_cta;
   uint32_t smem_bytes_per_cta;
   uint32_t t_in_smem;        /* 1: duplication (T) columns live in shared memory, 0: in global scratch */
-  uint32_t table_in_smem;    /* 1: each CTA keeps its slice of the transition table in shared memory */
+  uint32_t table_in_smem;    /* 1: each CTA keeps its out-table (its slice of the transition table) in shared memory */
   uint32_t s_prev_in_smem;   /* 1: the previous column S(pos-1) is in shared memory, 0: in L2-resident global scratch */
   uint32_t n_clusters;       /* clusters resident at once = reads in flight */
   uint32_t sm_count;
 } dnab_decoder_info;
 int dnab_decoder_get_info(const dnab_decoder* d, dnab_decoder_info* info);
 
-/* Tuning overrides (0 = automatic); must be set before the first batch. */
+/* Tuning overrides of the one-read-per-cluster kernel (0 = automatic; t_in_smem_mode 1 shared memory, 2 global scratch),
+ * the same as the options "cluster_size", "threads_per_cta" and "t_columns" below; must be set before the first batch. */
 int dnab_decoder_configure(dnab_decoder* d, uint32_t cluster_size, uint32_t threads_per_cta, uint32_t t_in_smem_mode);
-/* block_table_mode: units digit 0 auto, 1 transition table in shared memory, 2 in global memory;
- * tens digit 0 auto, 1 previous column S(pos-1) in shared memory, 2 in global scratch;
- * partition_mode: 0/1 equal runs of the reference state order + in-degree sort inside a CTA (default),
- * 2 runs of a depth-first order, unsorted, 3 DFS chunks dealt round-robin + sort, 4 DFS runs + sort. */
-int dnab_decoder_configure_ex(dnab_decoder* d, uint32_t block_table_mode, uint32_t partition_mode);
 
-/* Named options (replace the digit-encoded arguments above and every environment hook); set before the first batch.
+/* Named options; set before the first batch.
  *   "kernel"          0 automatic (read-batched when the machine fits, else one read per cluster), 1 read-batched
- *                     (viterbi_fill_batch.cu), 2 push closure, one read per cluster (viterbi_fill_push.cu), 3 pull closure
+ *                     (viterbi_fill_batch.cu), 2 push closure, one read per cluster (viterbi_fill_push.cu); 3, the
+ *                     pull-closure kernel of round 1, was retired and returns DNAB_EINVAL
  *   "team_size"       read-batched kernel: CTAs holding one group of 32 reads (0 = smallest that fits)
  *   "warps_per_cta"   read-batched kernel: 8, 16 or 32
  *   "cluster_size", "threads_per_cta", "t_columns" (1 shared / 2 global), "table" (1 shared / 2 global),
- *   "s_prev" (1 shared / 2 global), "partition" (1 index runs, 2 DFS runs, 3 DFS chunks dealt, 4 DFS runs sorted):
- *                     one-read-per-cluster kernels, as dnab_decoder_configure / _configure_ex
- *   "thin_n", "t_recompute", "queue_cap", "deal_chunks", "idle_sleep_ns": schedule knobs of the push kernel (tests)
- *   "async_closure"   read-batched kernel: 0 breadth-first levels with a CTA barrier each, 1 no level barriers (work counter), 2 (default)
- *                     automatic = 1 in a team, 0 in a single CTA; "batch_idle_ns" back-off of an idle warp; "team_slack_pct"
+ *   "s_prev" (1 shared / 2 global), "partition" (0 automatic = 3; 1 index runs, 2 DFS runs, 3 DFS chunks dealt,
+ *                     4 DFS runs sorted): placements of the one-read-per-cluster push kernel; setting any of them (or
+ *                     dnab_decoder_configure) makes "kernel" 0 choose the push kernel
+ *   "thin_n", "t_recompute", "queue_cap", "deal_chunks": schedule knobs of the push kernel (tests)
+ *   "idle_sleep_ns"   accepted and ignored (it tuned the retired pull-closure kernel)
+ *   "async_closure"   read-batched kernel: 0 breadth-first levels with a CTA barrier each, 1 no level barriers (work counter),
+ *                     2 (default) automatic = 1, in a team and in a single CTA alike; "batch_idle_ns" back-off of an idle warp;
+ *                     "team_slack_pct"
  *   "notify_classes"  read-batched kernel, teams: notification counters per CTA, 1..32 (default 32).  The states of a CTA that have
  *                     transitions from other CTAs are dealt into that many classes; a publishing state notifies the classes of its
  *                     successors and the owner re-relaxes only the notified classes (1 = every transition that crosses CTAs)

@@ -62,43 +62,51 @@ def test_gpu_every_cluster_size(d, name, cluster):
         _check_against_golden(d, case, dict(cluster_size=cluster, t_in_smem_mode=tmode))
 
 
-@pytest.mark.parametrize("cluster,table_mode,partition", [(3, 20, 0), (6, 20, 4), (8, 22, 3), (2, 21, 2), (1, 20, 0), (5, 12, 4)])
+# "table" / "s_prev": 1 shared memory, 2 global memory; "partition": 1 index runs, 2 DFS runs, 3 DFS chunks dealt,
+# 4 DFS runs sorted; 0 = automatic
+@pytest.mark.parametrize("cluster,table,s_prev,partition", [(3, 0, 2, 0), (6, 0, 2, 4), (8, 2, 2, 3), (2, 1, 2, 2), (1, 0, 2, 0),
+                                                           (5, 2, 1, 4), (4, 2, 2, 1), (12, 1, 1, 3), (16, 1, 1, 4)])
 @pytest.mark.parametrize("name", ["l4c4_local_mixed", "cfg3_global_indels", "cfg4_global_dels"])
-def test_gpu_memory_placements_and_partitions(d, name, cluster, table_mode, partition):
-    """S(pos-1) in global scratch, transition table in shared / global memory, odd cluster sizes and
-    every partition policy: none of it may change a bit."""
+def test_gpu_push_placements_and_partitions(d, name, cluster, table, s_prev, partition):
+    """S(pos-1) in shared memory / global scratch, transition table in shared / global memory, odd cluster sizes and
+    every partition policy of the push kernel, set through the named options: none of it may change a bit."""
     case = util.golden_case(name)
     if cluster == 1 and util.compiled_for_case(case).t.n_states > 4000:
         pytest.skip("does not fit one CTA")
+    opts = dict(table=table, s_prev=s_prev, partition=partition)
     try:
-        _check_against_golden(d, case, dict(cluster_size=cluster, table_mode=table_mode, partition_mode=partition))
+        _check_against_golden(d, case, dict(cluster_size=cluster), {k: v for k, v in opts.items() if v})
     except d.DnabError as e:
         if "does not fit" in str(e):
             pytest.skip("requested placement does not fit this machine")
         raise
 
 
-@pytest.mark.parametrize("name", ["l4c4_global_mixed", "l4c4_local_mixed", "cfg2_global_subs", "cfg3_global_indels", "cfg4_global_dels"])
-def test_gpu_pull_kernel_same_bits(d, name):
-    """The first fill kernel (pull-style closure, viterbi_kernels.cu; partition_mode tens digit 1) stays
-    selectable and must give the same bits as the push kernel that is now the default."""
-    _check_against_golden(d, util.golden_case(name), dict(partition_mode=10))
+def test_gpu_retired_pull_kernel_is_refused(d):
+    """kernel=3 selected the pull-closure fill kernel, which was retired: the option is refused with an error that
+    says so, and the handle keeps decoding with what it had."""
+    case = util.golden_case("l4c4_global_mixed")
+    dec = d.Decoder(util.compiled_for_case(case), device=0)
+    dec.set_option("kernel", 2)
+    with pytest.raises(d.DnabError, match="retired"):
+        dec.set_option("kernel", 3)
+    _check_reads(d, dec, case, "after kernel=3")
 
 
 @pytest.mark.parametrize("workload,n", [("cfg2", 99), ("cfg5", 300), ("cfg3", 300)])
-def test_gpu_two_kernels_agree_at_batch_scale(d, workload, n):
-    """Two independent implementations of the fill (push-style and pull-style closure, different table
-    formats, different cluster sizes) must agree bit for bit -- log-likelihood, decoded string, traceback
-    path -- on a batch far larger than the oracle can check in a test (several waves of clusters, ragged
+def test_gpu_fill_kernels_agree_at_batch_scale(d, workload, n):
+    """Two independent implementations of the fill (read-batched and one-read-per-cluster push kernel, different
+    table formats, different partitions) must agree bit for bit -- log-likelihood, decoded string, traceback
+    path -- on a batch far larger than the oracle can check in a test (several waves of clusters or teams, ragged
     lengths, dynamic read scheduling)."""
     import bench
     w = bench.WORKLOADS[workload]
     compiled = util.machine_from_recipe(w["recipe"]).compile(d.ErrorFlags(length=w["length"], global_=True))
     reads = bench.make_reads(w, n, seed=4242)
     outs = []
-    for part in (0, 10):
+    for kern in (1, 2):
         dec = d.Decoder(compiled, device=0)
-        dec.configure(partition_mode=part)
+        dec.set_option("kernel", kern)
         outs.append(dec.viterbi(reads, want_path=True))
     a, b = outs
     assert (a["status"] == 0).all() and (b["status"] == 0).all()
@@ -111,7 +119,8 @@ def test_gpu_two_kernels_agree_at_batch_scale(d, workload, n):
 
 @pytest.mark.parametrize("opts", [dict(thin_n=0), dict(thin_n=48), dict(t_recompute=0),
                                   dict(queue_cap=40), dict(queue_cap=40, thin_n=100000)])
-@pytest.mark.parametrize("name", ["l4c4_global_mixed", "cfg3_global_indels", "cfg4_global_dels", "cfg2_global_subs"])
+@pytest.mark.parametrize("name", ["l4c4_global_mixed", "l4c4_local_mixed", "cfg3_global_indels", "cfg4_global_dels",
+                                  "cfg2_global_subs"])
 def test_gpu_push_kernel_tuning_knobs_same_bits(d, name, opts):
     """How a level's work list is made (bitmap scan, or appended by the previous level's pushers below a size
     threshold -- including a threshold so large that the small append queues overflow), stored (not re-derived)

@@ -5,10 +5,12 @@ import numpy as np
 import bench, dnab_testutil as util, dnastore_b200 as d
 wl = sys.argv[1] if len(sys.argv) > 1 else 'cfg2'
 n = int(sys.argv[2]) if len(sys.argv) > 2 else 15
-cfg = ([int(x) for x in sys.argv[3:8]] + [0] * 5)[:5]
+cfg = ([int(x) for x in sys.argv[3:9]] + [0] * 6)[:6]  # cluster_size threads_per_cta t_columns table s_prev partition (0 = auto)
 w = bench.WORKLOADS[wl]
 m = util.machine_from_recipe(w['recipe']); c = m.compile(d.ErrorFlags(length=w['length'], global_=True))
-dec = d.Decoder(c); dec.configure(cfg[0], cfg[1], cfg[2], cfg[3], cfg[4])
+dec = d.Decoder(c); dec.configure(cfg[0], cfg[1], cfg[2])
+for key, v in zip(("table", "s_prev", "partition"), cfg[3:]):
+    if v: dec.set_option(key, v)
 reads = bench.make_reads(w, n, 7)
 dec.viterbi(reads[:2])
 dec.set_debug(True)
