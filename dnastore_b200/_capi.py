@@ -60,7 +60,7 @@ class DecoderInfo(C.Structure):
 
 class BatchInfo(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in ("enabled", "reads_per_group", "team_size", "states_per_cta", "warps_per_cta",
-                                          "smem_bytes_per_cta", "n_teams", "reserved")] + [("cross_cta_transition_fraction", C.c_double)]
+                                          "smem_bytes_per_cta", "n_teams", "wide_states")] + [("cross_cta_transition_fraction", C.c_double)]
 
 
 class PipelineStats(C.Structure):

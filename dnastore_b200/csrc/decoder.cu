@@ -97,7 +97,7 @@ struct dnab_decoder {
   DevBuf<uint4> dOutSlots;
   DevBuf<uint8_t> dSymChar;
   // scratch
-  DevBuf<uint8_t> dPred;
+  DevBuf<uint8_t> dPred, dPredWide;  // predecessor records; high bytes of the wide states' records (viterbi_device.cuh)
   DevBuf<double> dTScratch, dSScratch, dS0Scratch, dPartVal, dCells;
   DevBuf<uint32_t> dStart, dPartOrig, dPartG;
   DevBuf<unsigned long long> dDbg, dNextRead;
@@ -129,7 +129,8 @@ struct dnab_decoder {
   BatchTraceTables btrace{};
   DevBuf<uint4> dbHdr;
   DevBuf<uint2> dbIn, dbRel, dbHdr2;
-  DevBuf<uint32_t> dbOut, dbRankInOff, dbRankOutOff, dbRemoteIn, dbEmitOff, dbEmitSrc, dbNullOff, dbNullSrc, dbTeamState, dbTeamPassive, dbClsOff, dbClsStates, dbPartOrig;
+  DevBuf<uint32_t> dbOut, dbRankInOff, dbRankOutOff, dbRemoteIn, dbEmitOff, dbEmitSrc, dbNullOff, dbNullSrc, dbTeamState, dbTeamPassive, dbClsOff, dbClsStates, dbPartOrig, dbWideOf;
+  DevBuf<uint4> dbWide;
   DevBuf<uint8_t> dbEmitSym, dbNullSym;
   DevBuf<double> dbTsE, dbPriv, dbPartVal;
   DevBuf<double2> dbSdPub;
@@ -151,6 +152,33 @@ struct dnab_decoder {
 };
 
 namespace dnab {
+
+// Wide states (viterbi_device.cuh), numbered in reference order: wideOf[s] is the wide number of state s or 0xFFFFFFFF.
+// Refuses a state whose records or counts no format holds.  Both planners use this one classification.
+static int numberWideStates(const dnab_decoder* d, std::vector<uint32_t>& wideOf, uint32_t& nWide) {
+  const uint32_t N = d->nStates;
+  std::vector<uint32_t> nOut(N, 0);
+  for (uint32_t s : d->emitSrc) ++nOut[s];
+  for (uint32_t s : d->nullSrc) ++nOut[s];
+  wideOf.assign(N, 0xFFFFFFFFu);
+  nWide = 0;
+  for (uint32_t s = 0; s < N; ++s) {
+    const uint64_t nE = d->emitOff[s + 1] - d->emitOff[s], nN = d->nullOff[s + 1] - d->nullOff[s];
+    if (nE + nN + 3 > kMaxWideCandidates || 2 * nE + nN > kMaxWideCandidates) {
+      setLastError("state " + std::to_string(s) + " has " + std::to_string(nE) + " emitting and " + std::to_string(nN) +
+                   " null incoming transitions: predecessor records hold at most 65535 candidates (nEmit + nNull + 3 and "
+                   "2*nEmit + nNull must not exceed 65535)");
+      return DNAB_EINVAL;
+    }
+    if (nOut[s] > kMaxOutDegree) {
+      setLastError("state " + std::to_string(s) + " has " + std::to_string(nOut[s]) +
+                   " outgoing transitions: at most 65535 are supported");
+      return DNAB_EINVAL;
+    }
+    if (stateIsWide((uint32_t)nE, (uint32_t)nN, nOut[s])) wideOf[s] = nWide++;
+  }
+  return DNAB_OK;
+}
 
 // Alternative order of the states: depth-first preorder over the transition graph.  Cutting it
 // into C equal runs keeps more transitions inside one CTA (85% on the BASELINE config 2 machine
@@ -203,7 +231,7 @@ struct Partition {
   std::vector<uint32_t> blocks, blockOff;
 };
 
-static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
+static int buildPartition(const dnab_decoder* d, uint32_t C, const std::vector<uint32_t>& wideOf, Partition& P) {
   const uint32_t N = d->nStates, k = d->k;
   const uint32_t M = (N + C - 1) / C, Np = C * M;
   P.C = C;
@@ -267,7 +295,7 @@ static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
         const uint32_t nIn0 = (d->emitOff[s0 + 1] - d->emitOff[s0]) + (d->nullOff[s0 + 1] - d->nullOff[s0]);
         std::vector<uint32_t> tmp = outs[s0];
         std::sort(tmp.begin(), tmp.end());
-        words = 2 + 2 * nIn0 + (uint32_t)(std::unique(tmp.begin(), tmp.end()) - tmp.begin());
+        words = 2 + 2 * nIn0 + (uint32_t)(std::unique(tmp.begin(), tmp.end()) - tmp.begin()) + (wideOf[s0] != 0xFFFFFFFFu ? 2 : 0);
       }
       const uint32_t at = (uint32_t)P.blocks.size() % 8;
       if (words <= 8 && at + words > 8)
@@ -280,21 +308,20 @@ static int buildPartition(const dnab_decoder* d, uint32_t C, Partition& P) {
       P.blocks.push_back(0);
     } else {
       const uint32_t nE = d->emitOff[s + 1] - d->emitOff[s], nN = d->nullOff[s + 1] - d->nullOff[s];
-      if (nE > 126 || 2 * nE + nN > 254 || nE + nN + 2 > 254) {
-        setLastError("state " + std::to_string(s) + " has too many incoming transitions for 1-byte predecessor records");
-        return DNAB_EINVAL;
-      }
       auto& o = outs[s];
       std::sort(o.begin(), o.end());
       o.erase(std::unique(o.begin(), o.end()), o.end());
-      if (o.size() > 255) {
-        setLastError("state " + std::to_string(s) + " has more than 255 distinct successors");
-        return DNAB_EINVAL;
-      }
       uint32_t w1 = 0;
       for (uint32_t i = 0; i < d->mdl[s]; ++i) w1 |= (uint32_t)(d->ctx[(size_t)s * k + i] & 3u) << (2 * i);
-      P.blocks.push_back(nE | ((nE + nN) << 8) | ((uint32_t)o.size() << 16) | ((uint32_t)d->mdl[s] << 24));
-      P.blocks.push_back(w1);
+      if (wideOf[s] == 0xFFFFFFFFu) {
+        P.blocks.push_back(nE | ((nE + nN) << 8) | ((uint32_t)o.size() << 16) | ((uint32_t)d->mdl[s] << 24));
+        P.blocks.push_back(w1);
+      } else {
+        P.blocks.push_back(kHdrWide | ((uint32_t)d->mdl[s] << 24));
+        P.blocks.push_back(w1);
+        P.blocks.push_back(nE | ((nE + nN) << 16));
+        P.blocks.push_back(wideOf[s]);
+      }
       auto pushIn = [&](uint32_t src, uint32_t sym, uint32_t base) {
         const uint32_t sg = P.newOf[src], sr = sg / M;
         P.blocks.push_back(((sg % M) * 8) | (sr << 20) | (sr != rank ? kEdgeRemote : 0u));
@@ -316,7 +343,8 @@ struct PushTables {
   std::vector<uint4> outSlots;
 };
 
-static int buildPushTables(const dnab_decoder* d, const Partition& P, uint32_t chunkStates, PushTables& T) {
+static int buildPushTables(const dnab_decoder* d, const Partition& P, const std::vector<uint32_t>& wideOf, uint32_t chunkStates,
+                           PushTables& T) {
   const uint32_t threads = chunkStates;  // (states per chunk = kPushStatesPerThread * threads per CTA)
   const uint32_t N = d->nStates, k = d->k, C = P.C, M = P.M, Np = C * M;
   std::vector<std::vector<uint32_t>> outs(Np);  // out-edge words, "other CTA" bit added below
@@ -354,9 +382,15 @@ static int buildPushTables(const dnab_decoder* d, const Partition& P, uint32_t c
           continue;
         }
         const uint32_t nE = d->emitOff[s + 1] - d->emitOff[s], nN = d->nullOff[s + 1] - d->nullOff[s];
-        uint32_t h = nE | ((nE + nN) << 7) | ((uint32_t)d->mdl[s] << 15) | ((uint32_t)hasNullOut[s] << 30);
+        const bool wide = wideOf[s] != 0xFFFFFFFFu;
+        uint32_t h = (wide ? kInWide << 7 : nE | ((nE + nN) << 7)) | ((uint32_t)d->mdl[s] << 15) | ((uint32_t)hasNullOut[s] << 30);
         for (uint32_t i2 = 0; i2 < d->mdl[s]; ++i2) h |= (uint32_t)(d->ctx[(size_t)s * k + i2] & 3u) << (18 + 2 * i2);
         T.inChunks.push_back(h);
+        if (wide) {
+          T.inChunks.push_back(nE | ((nE + nN) << 16));
+          T.inChunks.push_back(wideOf[s]);
+          at += 2;
+        }
         auto pushIn = [&](uint32_t src, uint32_t sym, uint32_t base) {
           const uint32_t sg = P.newOf[src];
           T.inChunks.push_back(peMake(sg % M, sg / M, sg / M != r, sym, base));
@@ -442,6 +476,10 @@ static int buildPlan(dnab_decoder* d, int32_t maxLen) {
   LaunchPlan best;
   Partition P;
   PushTables T;
+  std::vector<uint32_t> wideOf;
+  uint32_t nWide = 0;
+  int wrc = numberWideStates(d, wideOf, nWide);
+  if (wrc != DNAB_OK) return wrc;
   std::vector<uint32_t> cands = {1, 2, 3, 4, 5, 6, 7, 8, 10, 12, 14, 16};
   if (d->wantC >= 1 && d->wantC <= (uint32_t)kMaxCluster) cands = {d->wantC};
   // Preference: the smallest cluster whose CTAs hold S and D (more reads in flight beats more SMs per
@@ -454,9 +492,9 @@ static int buildPlan(dnab_decoder* d, int32_t maxLen) {
     if (M > 65535) continue;
     const uint32_t threads = pushThreads(d, M);
     if (makePushLayout(M, k, 0, 0, 0, 64, 1, (uint32_t)planLen, 1024).total > d->smemOptin) continue;
-    int rc = buildPartition(d, C, P);
+    int rc = buildPartition(d, C, wideOf, P);
     if (rc != DNAB_OK) return rc;
-    rc = buildPushTables(d, P, threads * kPushStatesPerThread, T);
+    rc = buildPushTables(d, P, wideOf, threads * kPushStatesPerThread, T);
     if (rc != DNAB_OK) {
       if (d->wantC) return rc;
       continue;
@@ -509,6 +547,7 @@ static int buildPlan(dnab_decoder* d, int32_t maxLen) {
   t.startG = P.newOf[0];
   t.endG = P.newOf[N - 1];
   t.tInSmem = best.tInSmem;
+  t.nWide = nWide;
   t.sPrevInSmem = best.sPrevGlobal ? 0 : 1;
   t.outInSmem = best.outInSmem;
   t.chunkStates = T.chunkStates;
@@ -685,12 +724,11 @@ static int buildBatchPlan(dnab_decoder* d) {
   uint32_t W = wantW ? wantW : 24u;
   auto nEmitOf = [&](uint32_t s) { return d->emitOff[s + 1] - d->emitOff[s]; };
   auto nNullOf = [&](uint32_t s) { return d->nullOff[s + 1] - d->nullOff[s]; };
-  for (uint32_t s = 0; s < N; ++s) {
-    const uint32_t nE = nEmitOf(s), nN = nNullOf(s);
-    if (nE > 126 || 2 * nE + nN > 254 || nE + nN + 2 > 254) {
-      setLastError("state " + std::to_string(s) + " has too many incoming transitions for 1-byte predecessor records");
-      return DNAB_EINVAL;
-    }
+  std::vector<uint32_t> wideOf;
+  uint32_t nWide = 0;
+  {
+    const int rc = numberWideStates(d, wideOf, nWide);
+    if (rc != DNAB_OK) return rc;
   }
   // successors of every state with the bit they own in the successor's work mask
   std::vector<std::vector<std::pair<uint32_t, uint32_t>>> outs(N);
@@ -699,16 +737,11 @@ static int buildBatchPlan(dnab_decoder* d) {
     for (uint32_t e = d->emitOff[dst]; e < d->emitOff[dst + 1]; ++e, ++j) outs[d->emitSrc[e]].push_back({dst, j});
     for (uint32_t e = d->nullOff[dst]; e < d->nullOff[dst + 1]; ++e, ++j) outs[d->nullSrc[e]].push_back({dst, j});
   }
-  for (auto& o : outs)
-    if (o.size() > 255) {
-      setLastError("a state has more than 255 outgoing transitions");
-      return DNAB_EINVAL;
-    }
   const std::vector<uint32_t> dfs = dfsOrder(d);
   const uint32_t nSymsB = (uint32_t)d->symChar.size();
   const uint32_t maxTeam = (uint32_t)d->smCount;
   uint32_t T0 = std::max<uint32_t>(1, (uint32_t)(((size_t)N * kBatchReads * 16 + d->smemOptin - 1) / d->smemOptin));
-  std::vector<uint4> hdr;
+  std::vector<uint4> hdr, wideHdr(nWide);
   std::vector<uint2> inE, relE, hdr2;
   std::vector<uint32_t> outE, rankInOff, rankOutOff, newOf(N), origOf, remoteIn, clsOff, clsStates, clsOf;
   // builds the tables of a team of T CTAs; false when T is infeasible
@@ -818,7 +851,12 @@ static int buildBatchPlan(dnab_decoder* d) {
             relE[base + relPos[s][j]] = make_uint2(newOf[src], sym * 8);
             if (remote) remoteIn[r * M + i] |= 1u << std::min(relPos[s][j], 31u);
           }
-          hdr2[r * M + i] = make_uint2(base - rankInOff[r], cnt[0] | (cnt[1] << 8) | (cnt[2] << 16) | (cnt[3] << 24));
+          if (wideOf[s] == 0xFFFFFFFFu)
+            hdr2[r * M + i] = make_uint2(base - rankInOff[r], cnt[0] | (cnt[1] << 8) | (cnt[2] << 16) | (cnt[3] << 24));
+          else {
+            hdr2[r * M + i] = make_uint2(base - rankInOff[r], 0);
+            wideHdr[wideOf[s]] = make_uint4(nE | (nN << 16), cnt[0] | (cnt[1] << 16), cnt[2] | (cnt[3] << 16), 0);
+          }
         }
         bool remoteOut = (d->local && s == 0 && T > 1);  // local mode: every CTA reads S(start,0) for the (0,0) escape
         uint32_t nLocal = 0;
@@ -837,12 +875,17 @@ static int buildBatchPlan(dnab_decoder* d) {
         std::sort(remoteNotes.begin(), remoteNotes.end());
         remoteNotes.erase(std::unique(remoteNotes.begin(), remoteNotes.end()), remoteNotes.end());
         outE.insert(outE.end(), remoteNotes.begin(), remoteNotes.end());
-        const uint32_t nOutEntries = nLocal + (uint32_t)remoteNotes.size();
-        if (nOutEntries > 255) return false;
+        const uint32_t nOutEntries = nLocal + (uint32_t)remoteNotes.size();  // (<= outgoing transitions: 255 when narrow)
         uint32_t ctxBits = 0;
         for (uint32_t t = 0; t < d->mdl[s]; ++t) ctxBits |= (uint32_t)(d->ctx[(size_t)s * k + t] & 3u) << (2 * t);
-        hdr[r * M + i] = make_uint4(inOff | (outOff << 16), nE | (nN << 8) | (nOutEntries << 16) | ((uint32_t)d->mdl[s] << 24),
-                                    ctxBits | (remoteOut ? 1u << 16 : 0u) | (nLocal << 18), s);
+        if (wideOf[s] == 0xFFFFFFFFu)
+          hdr[r * M + i] = make_uint4(inOff | (outOff << 16), nE | (nN << 8) | (nOutEntries << 16) | ((uint32_t)d->mdl[s] << 24),
+                                      ctxBits | (remoteOut ? 1u << 16 : 0u) | (nLocal << 18), s);
+        else {
+          hdr[r * M + i] = make_uint4(inOff | (outOff << 16), wideOf[s] | ((uint32_t)d->mdl[s] << 24) | kBhWide,
+                                      ctxBits | (remoteOut ? 1u << 16 : 0u), s);
+          wideHdr[wideOf[s]].w = nLocal | (nOutEntries << 16);
+        }
       }
       maxIn = std::max(maxIn, (uint32_t)inE.size() - rankInOff[r]);
       maxOut = std::max(maxOut, (uint32_t)outE.size() - rankOutOff[r]);
@@ -956,6 +999,10 @@ static int buildBatchPlan(dnab_decoder* d) {
   CUDA_TRY(d->dbClsOff.upload(clsOff));
   CUDA_TRY(d->dbClsStates.upload(clsStates));
   CUDA_TRY(d->dbTsE.upload(tsE));
+  if (nWide) {
+    CUDA_TRY(d->dbWide.upload(wideHdr));
+    CUDA_TRY(d->dbWideOf.upload(wideOf));
+  }
   // traceback tables in reference order
   CUDA_TRY(d->dbEmitOff.upload(d->emitOff));
   CUDA_TRY(d->dbEmitSrc.upload(d->emitSrc));
@@ -994,11 +1041,15 @@ static int buildBatchPlan(dnab_decoder* d) {
   t.hdr2 = d->dbHdr2.p;
   t.relEdges = d->dbRel.p;
   t.tsE = d->dbTsE.p;
+  t.nWide = nWide;
+  t.wide = nWide ? d->dbWide.p : nullptr;
   BatchTraceTables tt{};
   tt.nStates = N;
   tt.k = k;
   tt.local = d->local;
   tt.T = bp.T * bp.warps;
+  tt.nWide = nWide;
+  tt.wideOf = nWide ? d->dbWideOf.p : nullptr;
   tt.emitOff = d->dbEmitOff.p;
   tt.emitSrc = d->dbEmitSrc.p;
   tt.emitSym = d->dbEmitSym.p;
@@ -1042,10 +1093,12 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
   const BatchPlan& bp = d->bplan;
   const uint32_t N = d->nStates, K2 = d->k + 2;
   const int64_t nGroups = (nReads + 31) / 32;
+  const size_t perGroupWide = (size_t)(maxLen + 1) * d->btab.nWide * 2 * 32;  // the side plane (wide states only)
   const size_t perGroup = (size_t)(maxLen + 1) * N * K2 * 32;
-  int64_t chunk = (int64_t)std::max<size_t>(1, d->predBudgetBytes / perGroup);
+  int64_t chunk = (int64_t)std::max<size_t>(1, d->predBudgetBytes / (perGroup + perGroupWide));
   chunk = std::min<int64_t>(chunk, nGroups);
   CUDA_TRY(d->dPred.ensure((size_t)chunk * perGroup));
+  if (perGroupWide) CUDA_TRY(d->dPredWide.ensure((size_t)chunk * perGroupWide));
   if (d->local) {
     CUDA_TRY(d->dbPartVal.ensure((size_t)chunk * bp.T * bp.warps * 32));
     CUDA_TRY(d->dbPartOrig.ensure((size_t)chunk * bp.T * bp.warps * 32));
@@ -1077,6 +1130,7 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
     a.readLen = dReadLen;
     a.order = dOrder ? dOrder + at * 32 : nullptr;
     a.pred = d->dPred.p;
+    a.predWide = perGroupWide ? d->dPredWide.p : nullptr;
     a.priv = d->dbPriv.p;
     a.sdPub = d->dbSdPub.p;
     a.teamState = d->dbTeamState.p;
@@ -1107,6 +1161,7 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
     ta.nReads = nReads;
     ta.readBase = a.readBase;
     ta.pred = d->dPred.p;
+    ta.predWide = a.predWide;
     ta.loglike = dLoglike;
     ta.partVal = d->dbPartVal.p;
     ta.partOrig = d->dbPartOrig.p;
@@ -1130,6 +1185,7 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
 static size_t predBytesPerRead(const dnab_decoder* d, int32_t maxLen) {
   return (size_t)(maxLen + 1) * (d->k + 2) * (size_t)d->plan.C * d->plan.M;
 }
+static size_t predWideBytesPerRead(const dnab_decoder* d, int32_t maxLen) { return (size_t)(maxLen + 1) * 2 * d->dev.nWide; }
 
 // fill + traceback over device-resident inputs/outputs, chunked so that the
 // predecessor records of one chunk fit the scratch budget
@@ -1155,10 +1211,11 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
   }
   int rc = buildPlan(d, maxLen);
   if (rc != DNAB_OK) return rc;
-  const size_t perRead = predBytesPerRead(d, maxLen);
-  int64_t chunk = (int64_t)std::max<size_t>(1, d->predBudgetBytes / perRead);
+  const size_t perRead = predBytesPerRead(d, maxLen), perReadWide = predWideBytesPerRead(d, maxLen);
+  int64_t chunk = (int64_t)std::max<size_t>(1, d->predBudgetBytes / (perRead + perReadWide));
   chunk = std::min<int64_t>(chunk, nReads);
   CUDA_TRY(d->dPred.ensure((size_t)chunk * perRead));
+  if (perReadWide) CUDA_TRY(d->dPredWide.ensure((size_t)chunk * perReadWide));
   CUDA_TRY(d->dStart.ensure((size_t)chunk));
   if (d->local) {
     CUDA_TRY(d->dPartVal.ensure((size_t)chunk * d->plan.C));
@@ -1178,6 +1235,7 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
     fa.byteOff = dByteOff + at;
     fa.readLen = dReadLen + at;
     fa.pred = d->dPred.p;
+    fa.predWide = perReadWide ? d->dPredWide.p : nullptr;
     fa.tScratch = d->dTScratch.p;
     fa.sScratch = d->dSScratch.p;
     fa.s0Scratch = d->dS0Scratch.p;
@@ -1203,6 +1261,7 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
     ta.maxLen = maxLen;
     ta.readLen = dReadLen + at;
     ta.pred = d->dPred.p;
+    ta.predWide = fa.predWide;
     ta.loglike = dLoglike + at;
     ta.startState = d->dStart.p;
     ta.partVal = d->dPartVal.p;
@@ -1426,6 +1485,7 @@ int dnab_decoder_get_batch_info(const dnab_decoder* dc, dnab_batch_info* info) {
   info->smem_bytes_per_cta = d->bplan.smemBytes;
   info->n_teams = d->bplan.nTeams;
   info->cross_cta_transition_fraction = d->bplan.crossFraction;
+  info->wide_states = d->btab.nWide;
   return DNAB_OK;
 }
 

@@ -44,6 +44,11 @@ constexpr uint32_t kBatchAllEdges = 0xFFFFFFFFu;
 //                   y: local emit | local null << 8 | remote emit << 16 | remote null << 24   (counts, in this order)
 //   relax   uint2   x: padded index g of the source, y: symbol id * 8 (byte offset of its score)
 //   Bit j of a state's work mask is its j-th relax entry (31 = "31 or later").
+//   A WIDE state (viterbi_device.cuh) has bit 27 of header.y set and its wide number in bits 0..23 of header.y
+//   (mdl stays in bits 24..26); its counts are in the wide table instead of the 8-bit fields of header.y, header.z
+//   and hdr2.y:
+//   wide    uint4   x: nEmit | nNull << 16   y: local emit | local null << 16   z: remote emit | remote null << 16
+//                   w: nOutLocal | nOut << 16
 // ---------------------------------------------------------------------------
 __host__ __device__ inline uint32_t bhInOff(const uint4& h) { return h.x & 0xFFFFu; }
 __host__ __device__ inline uint32_t bhOutOff(const uint4& h) { return h.x >> 16; }
@@ -55,6 +60,9 @@ __host__ __device__ inline uint32_t bhCtx(const uint4& h, uint32_t i) { return (
 __host__ __device__ inline uint32_t bhRemoteOut(const uint4& h) { return (h.z >> 16) & 1u; }
 __host__ __device__ inline uint32_t bhPad(const uint4& h) { return (h.z >> 17) & 1u; }
 __host__ __device__ inline uint32_t bhNOutLocal(const uint4& h) { return (h.z >> 18) & 0xFFu; }
+constexpr uint32_t kBhWide = 1u << 27;
+__host__ __device__ inline uint32_t bhWide(const uint4& h) { return (h.y >> 27) & 1u; }
+__host__ __device__ inline uint32_t bhWideNo(const uint4& h) { return h.y & 0xFFFFFFu; }
 __host__ __device__ inline uint32_t beSym(const uint2& e) { return e.y & 31u; }
 __host__ __device__ inline uint32_t beBase(const uint2& e) { return (e.y >> 5) & 3u; }
 __host__ __device__ inline uint32_t beRemote(const uint2& e) { return (e.y >> 7) & 1u; }
@@ -81,6 +89,8 @@ struct BatchTables {
   const uint2* hdr2;             // [T*M]
   const uint2* relEdges;         // all ranks, rank r at rankInOff[r] (as many relax entries as in-edges)
   const double* tsE;             // [32 syms][4 bases][4 observed] (score+noGap)+sub: traceback association (src/viterbi.cpp:255)
+  const uint4* wide;             // [nWide] counts of the wide states
+  uint32_t nWide;
   double symScore[kMaxSyms];     // log(symProb) per symbol id (0 for id 0)
   double tsDext[kMaxSyms];       // score+delExtend (src/viterbi.cpp:272)
   double tsDopen[kMaxSyms];      // score+delOpen   (src/viterbi.cpp:273)
@@ -103,6 +113,7 @@ struct BatchArgs {
   const int32_t* readLen;        // [nReads]
   const int32_t* order;          // optional [nGroups*32]: slot -> read (-1 = empty lane); null = identity
   uint8_t* pred;                 // [nGroups][maxLen+1][nStates][k+2][32] predecessor records, 1 byte per DP cell, reference state order
+  uint8_t* predWide;             // [nGroups][maxLen+1][nWide][2][32] high bytes of the wide states' S and D records
   double* priv;                  // [nTeams][Np][2+k][32] rows private to the owning lane, carried from one column to the next:
                                  //   S0 of the next column (emission step fused into the record pass), the best emit candidate of
                                  //   its S record (traceback association), the k parked duplication cells
@@ -150,6 +161,8 @@ __host__ __device__ inline BatchLayout makeBatchLayout(uint32_t M, uint32_t maxI
 // reference-order CSR tables for the traceback over batch-layout records
 struct BatchTraceTables {
   uint32_t nStates, k, local, T;  // T = per-group partial maxima in local mode (CTAs x warps)
+  uint32_t nWide;
+  const uint32_t* wideOf;         // [nStates] wide number of every state (0xFFFFFFFF: narrow); null when nWide = 0
   const uint32_t* emitOff;
   const uint32_t* emitSrc;
   const uint8_t* emitSym;
@@ -167,6 +180,7 @@ struct BatchTraceArgs {
   int64_t nReads;
   int64_t readBase;
   const uint8_t* pred;
+  const uint8_t* predWide;
   double* loglike;
   const double* partVal;
   const uint32_t* partOrig;

@@ -11,6 +11,27 @@ constexpr int kMaxCluster = 16;
 constexpr uint32_t kNoPred = 255;  // predecessor record: "no candidate"
 
 // ---------------------------------------------------------------------------
+// Wide states.  A predecessor record is one byte: the index of the winning candidate in the state's
+// list (S: nE emit edges, nN null edges, delEnd, T -> S, local start; D: 2*nE emit candidates, nN null
+// ones; T: 2), 255 = none.  A state is WIDE when that byte, or one of the 7- and 8-bit count fields of
+// the narrow table headers, cannot hold it: nE > 126, nE + nN + 2 > 254 (largest S index), 2*nE + nN
+// > 254 (D candidates), or more than 255 outgoing transitions.  Narrow machines (no wide state) use
+// exactly the narrow formats.  The wide states of a machine are numbered 0 .. nWide-1 in reference
+// order; their S and D records keep the LOW byte in the ordinary record array and store the HIGH byte
+// in a side plane, one byte per (wide state, record kind) next to it:
+//   read-batched kernel  [group][pos][wide][2][32 reads]
+//   push kernel          [read][pos][2][nWide]
+// A wide record is the 16-bit index (high << 8 | low), 0xFFFF = none, so a wide state may have at
+// most 65,535 candidates in either record (kMaxWideCandidates).  T records stay narrow.
+// ---------------------------------------------------------------------------
+constexpr uint32_t kWideNoPred = 0xFFFFu;
+constexpr uint32_t kMaxWideCandidates = 65535;  // nE + nN + 3 (S) and 2*nE + nN (D)
+constexpr uint32_t kMaxOutDegree = 65535;       // outgoing transitions of one state (16-bit counts of the wide headers)
+__host__ __device__ inline bool stateIsWide(uint32_t nE, uint32_t nN, uint32_t nOut) {
+  return nE > 126 || nE + nN + 2 > 254 || 2 * nE + nN > 254 || nOut > 255;
+}
+
+// ---------------------------------------------------------------------------
 // State blocks: the traceback kernel decodes a predecessor record of state g against g's
 // block (the record is an index into g's incoming edges).  The padded state space (Np = C*M
 // states; state g lives in CTA rank g/M at local index g%M) is described by one block of
@@ -30,8 +51,12 @@ constexpr uint32_t kNoPred = 255;  // predecessor record: "no candidate"
 //              bits 0..15 local index, bits 20..23 rank, bit 24 "other CTA"
 //   padding to an even number of words.
 // Of these the traceback reads nEmit, nIn and the source and symbol of an incoming edge.
+// A wide state's block has nEmit = kHdrWide and two more words before its edges:
+//   word 2   nEmit | nIn << 16,   word 3   the state's wide number
+// (its nOut field is not used).
 // ---------------------------------------------------------------------------
 constexpr uint32_t kEdgeRemote = 1u << 24;
+constexpr uint32_t kHdrWide = 0xFFu;
 __host__ __device__ inline uint32_t hdrNEmit(uint32_t w0) { return w0 & 0xFFu; }
 __host__ __device__ inline uint32_t hdrNIn(uint32_t w0) { return (w0 >> 8) & 0xFFu; }
 __host__ __device__ inline uint32_t edgeOff(uint32_t a) { return a & 0xFFFFFu; }
@@ -50,6 +75,8 @@ __host__ __device__ inline uint32_t edgeSymOff(uint32_t b) { return b & 0xFFu; }
 //      record = header word, then nIn edge words (emit edges first, reference list order)
 //      header: bits 0..6 nEmit | 7..14 nIn (255 = padding state) | 15..17 mdl | 18..29 ctx
 //              (2 bits per duplication index) | 30 "has an outgoing null transition"
+//      a wide state has nIn = kInWide in its header and two more words before its edges:
+//              nEmit | nIn << 16, then its wide number
 //      edge:   bits 0..15 source's local index | 16..19 source's rank | 20 source in another
 //              CTA | 21..25 input-symbol id | 26..27 emitted base
 //  * OUT-TABLE, resident in shared memory when it fits.  The closure after the first pass is
@@ -59,6 +86,7 @@ __host__ __device__ inline uint32_t edgeSymOff(uint32_t b) { return b & 0xFFu; }
 //              21..25 input-symbol id | 26 transition emits a base
 // ---------------------------------------------------------------------------
 constexpr uint32_t kInPad = 255;
+constexpr uint32_t kInWide = 254;  // (a narrow state has nIn <= 252)
 __host__ __device__ inline uint32_t inNEmit(uint32_t h) { return h & 0x7Fu; }
 __host__ __device__ inline uint32_t inNIn(uint32_t h) { return (h >> 7) & 0xFFu; }
 __host__ __device__ inline uint32_t inMdl(uint32_t h) { return (h >> 15) & 0x7u; }
@@ -84,7 +112,8 @@ struct DevTables {
   uint32_t startG;    // padded-space index of reference state 0
   uint32_t endG;      // padded-space index of the reference's last state
   uint32_t tInSmem;   // T columns in shared memory (else in global scratch)
-  const uint32_t* blocks;     // state blocks (traceback)
+  uint32_t nWide;     // wide states (side plane entries per column and record kind)
+  const uint32_t* blocks;    // state blocks (traceback)
   const uint32_t* blockOff;   // [Np] word offset of each state's block
   const uint32_t* origId;     // [Np] reference state index, 0xFFFFFFFF for padding
   const uint8_t* symChar;     // [nSyms] input-symbol character of each id

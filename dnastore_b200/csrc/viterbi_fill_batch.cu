@@ -80,6 +80,7 @@ __device__ __forceinline__ unsigned long long ldAcquire64(const unsigned long lo
 
 enum : uint32_t { kCtlFlag = 0, kCtlWake = 4, kCtlDecision = 8, kCtlPending = 16, kCtlPhase = 17, kCtlLock = 18, kCtlSeen = 32 };
 constexpr uint32_t kKeepRecord = 0x100u;  // "the S record written by the previous column's pass stands"
+constexpr uint32_t kKeepRecordWide = 0x10000u;  // (the same in a kernel for wide states, whose indices reach 0xFFFF)
 
 __device__ __forceinline__ void fenceRelease() { asm volatile("fence.release.gpu;" ::: "memory"); }
 __device__ __forceinline__ void stRecordEarly(uint8_t* p, uint32_t v) { asm volatile("st.global.u8 [%0], %1;" ::"l"(p), "r"(v) : "memory"); }
@@ -107,8 +108,9 @@ __device__ __forceinline__ void stRelaxed32(uint32_t* p, uint32_t v) {
 
 }  // namespace
 
-// W warps per CTA; KMAX >= k duplication columns unrolled; kTeam: the group's states are spread over T > 1 CTAs.
-template <int W, int KMAX, bool kTeam, bool kDebug>
+// W warps per CTA; KMAX >= k duplication columns unrolled; kTeam: the group's states are spread over T > 1 CTAs;
+// kWide: the machine has wide states (viterbi_device.cuh, viterbi_batch.h); only those machines run this instantiation.
+template <int W, int KMAX, bool kTeam, bool kDebug, bool kWide>
 __global__ void __launch_bounds__(W * 32, 1)
     viterbiFillBatchKernel(const __grid_constant__ BatchTables tb, const __grid_constant__ BatchArgs args) {
   extern __shared__ __align__(16) unsigned char smem[];
@@ -119,6 +121,10 @@ __global__ void __launch_bounds__(W * 32, 1)
   const uint32_t nSlots = (M + W - 1) / W;
   const double NEG = negInf();
   const BatchLayout lay = makeBatchLayout(M, tb.maxIn, tb.maxOut, tb.nSyms, kTeam);
+  // counts of a wide state (header: viterbi_batch.h)
+  auto wideCounts = [&](const uint4& h) { return __ldg(tb.wide + bhWideNo(h)); };
+  auto nOutLocalOf = [&](const uint4& h) { return (kWide && bhWide(h)) ? (wideCounts(h).w & 0xFFFFu) : bhNOutLocal(h); };
+  auto nOutOf = [&](const uint4& h) { return (kWide && bhWide(h)) ? (wideCounts(h).w >> 16) : bhNOut(h); };
 
   const uint32_t aSD = smemAddr(smem + lay.sd);
   uint32_t* maskCur = reinterpret_cast<uint32_t*>(smem + lay.maskA);
@@ -158,7 +164,11 @@ __global__ void __launch_bounds__(W * 32, 1)
     __syncthreads();
     for (uint32_t i = tid; i < M; i += nThreads) {
       const uint2 h2 = hdr2S[i];
-      const uint32_t nLoc = (h2.y & 0xFFu) + ((h2.y >> 8) & 0xFFu);
+      uint32_t nLoc = (h2.y & 0xFFu) + ((h2.y >> 8) & 0xFFu);
+      if (kWide && bhWide(hdrS[i])) {
+        const uint32_t lc = wideCounts(hdrS[i]).y;
+        nLoc = (lc & 0xFFFFu) + (lc >> 16);
+      }
       for (uint32_t j = 0; j < nLoc; ++j) relS[h2.x + j].x = aSD + (relS[h2.x + j].x - rank * M) * 512u;
     }
     const uint32_t outBase = tb.rankOutOff[rank], nOut = tb.rankOutOff[rank + 1] - outBase;
@@ -218,6 +228,7 @@ __global__ void __launch_bounds__(W * 32, 1)
     int32_t Lmax = L;
     for (int sh = 16; sh > 0; sh >>= 1) Lmax = max(Lmax, __shfl_xor_sync(0xFFFFFFFFu, Lmax, sh));
     uint8_t* const predG = args.pred + (size_t)group * (size_t)(args.maxLen + 1) * N * K2 * 32;
+    uint8_t* const predWideG = kWide ? args.predWide + (size_t)group * (size_t)(args.maxLen + 1) * tb.nWide * 64 + lane : nullptr;
     unsigned long long win = 0;
     uint32_t xNext = 0;
 
@@ -280,7 +291,14 @@ __global__ void __launch_bounds__(W * 32, 1)
         const uint32_t d = sl * W + warp;
         const uint4 h = hdrS[d];
         const uint2 h2 = hdr2S[d];
-        const uint32_t nLE = h2.y & 0xFFu, nLN = (h2.y >> 8) & 0xFFu, nRE = (h2.y >> 16) & 0xFFu, nRN = h2.y >> 24;
+        uint32_t nLE = h2.y & 0xFFu, nLN = (h2.y >> 8) & 0xFFu, nRE = (h2.y >> 16) & 0xFFu, nRN = h2.y >> 24;
+        if (kWide && bhWide(h)) {
+          const uint4 wc = wideCounts(h);
+          nLE = wc.y & 0xFFFFu;
+          nLN = wc.y >> 16;
+          nRE = wc.z & 0xFFFFu;
+          nRN = wc.z >> 16;
+        }
         const uint32_t eLN = nLE + nLN, eRE = eLN + nRE, nIn = eRE + nRN;
         const uint2* const rel = relS + h2.x;
         const uint32_t aOwn = aSD + d * 512u + lane16;
@@ -358,7 +376,7 @@ __global__ void __launch_bounds__(W * 32, 1)
           stPub2(sdPubCol + (size_t)(rank * M + d) * 32 + lane, s, dd);
           remotePending |= 1u << sl;
         }
-        const uint32_t nLoc = bhNOutLocal(h), outOff = bhOutOff(h);
+        const uint32_t nLoc = nOutLocalOf(h), outOff = bhOutOff(h);
         uint32_t* const flagTo = asyncClosure ? maskCur : maskNext;
 #pragma unroll 1
         for (uint32_t o = lane; o < nLoc; o += 32) {
@@ -376,7 +394,7 @@ __global__ void __launch_bounds__(W * 32, 1)
         uint32_t nNotes = 0;
         for (uint32_t rp = remotePending; rp; rp &= rp - 1u) {
           const uint4 h = hdrS[((uint32_t)__ffs((int)rp) - 1u) * W + warp];
-          nNotes += bhNOut(h) - bhNOutLocal(h);
+          nNotes += nOutOf(h) - nOutLocalOf(h);
         }
         const bool eager = args.eagerNotify != 0;
         if (lane == 0) redAdd32(passiveCol, 0u - (eager ? 2u * nNotes : nNotes));
@@ -387,7 +405,7 @@ __global__ void __launch_bounds__(W * 32, 1)
           __syncwarp();
           for (uint32_t rp = remotePending; rp; rp &= rp - 1u) {
             const uint4 h = hdrS[((uint32_t)__ffs((int)rp) - 1u) * W + warp];
-            const uint32_t first = bhOutOff(h) + bhNOutLocal(h), last = bhOutOff(h) + bhNOut(h);
+            const uint32_t first = bhOutOff(h) + nOutLocalOf(h), last = bhOutOff(h) + nOutOf(h);
             for (uint32_t o = first + lane; o < last; o += 32) redAdd32(notifyT + outS[o], 1u);
           }
         }
@@ -397,7 +415,7 @@ __global__ void __launch_bounds__(W * 32, 1)
           const uint32_t sl = (uint32_t)__ffs((int)remotePending) - 1u;
           remotePending &= remotePending - 1u;
           const uint4 h = hdrS[sl * W + warp];
-          const uint32_t first = bhOutOff(h) + bhNOutLocal(h), last = bhOutOff(h) + bhNOut(h);
+          const uint32_t first = bhOutOff(h) + nOutLocalOf(h), last = bhOutOff(h) + nOutOf(h);
           for (uint32_t o = first + lane; o < last; o += 32) redAdd32(notifyT + outS[o], 1u);  // (owner CTA, class) of the successors
         }
       };
@@ -676,13 +694,22 @@ __global__ void __launch_bounds__(W * 32, 1)
           if (sl + 1 < nSlots) fetch(sl + 1);
           const uint4 h = hdrS[d];
           if (bhPad(h)) continue;
-          const uint32_t inOff = bhInOff(h), nE = bhNEmit(h), nIn = nE + bhNNull(h), mdl = bhMdl(h), orig = h.w;
+          const bool wide = kWide && bhWide(h);
+          uint32_t nE = bhNEmit(h), nIn = nE + bhNNull(h);
+          if (wide) {
+            const uint32_t c = wideCounts(h).x;
+            nE = c & 0xFFFFu;
+            nIn = nE + (c >> 16);
+          }
+          const uint32_t inOff = bhInOff(h), mdl = bhMdl(h), orig = h.w;
+          constexpr uint32_t keep = kWide ? kKeepRecordWide : kKeepRecord;
+          const uint32_t none = wide ? kWideNoPred : kNoPred;
           double* const row = privT + (size_t)(rank * M + d) * privKinds * 32;
           const double2 own = ldsRow(aSD + d * 512u + lane16);
           const double sH = own.x, dH = own.y;
           // S record: the emit candidates (:255) were evaluated by the previous column's pass
           double best = pos > 0 ? curB : NEG, bestD = NEG, s0n = NEG, bEn = NEG;
-          uint32_t idx = pos > 0 ? kKeepRecord : kNoPred, idxD = kNoPred, idxEn = kNoPred;
+          uint32_t idx = pos > 0 ? keep : none, idxD = none, idxEn = none;
           uint32_t j = 0;
 #pragma unroll 1
           for (; j < nE; ++j) {
@@ -747,9 +774,14 @@ __global__ void __launch_bounds__(W * 32, 1)
             }
           }
           uint8_t* const pr = predG + ((size_t)pos * N + orig) * K2 * 32 + lane;
+          uint8_t* const prW = wide ? predWideG + ((size_t)pos * tb.nWide + bhWideNo(h)) * 64 : nullptr;  // the high bytes
           if (act) {
-            if (idx != kKeepRecord) stRecord(pr, idx);
+            if (idx != keep) stRecord(pr, idx);
             stRecord(pr + 32, idxD);
+            if (wide) {
+              if (idx != keep) stRecord(prW, idx >> 8);
+              stRecord(prW + 32, idxD >> 8);
+            }
           }
           // duplication cells (:161-168) and their records (:281-286).  Parked layout between columns: slot 0 holds
           // T(pos,0)+sub (the T -> S candidate of the next column), slot t >= 1 holds T(pos,t)+sub (the shift into t-1).
@@ -789,7 +821,10 @@ __global__ void __launch_bounds__(W * 32, 1)
           }
           stCarried(row, s0n, polLast);
           stCarried(row + 32, bEn, polLast);
-          if (pos < L) stRecordEarly(pr + (size_t)N * K2 * 32, idxEn);  // the emit part of S(state,pos+1)'s record
+          if (pos < L) {  // the emit part of S(state,pos+1)'s record
+            stRecordEarly(pr + (size_t)N * K2 * 32, idxEn);
+            if (wide) stRecordEarly(prW + (size_t)tb.nWide * 64, idxEn >> 8);
+          }
           if (kTeam && bhRemoteOut(h)) stPub2(sdPubNext + (size_t)(rank * M + d) * 32 + lane, s0n, NEG);
           if (!tb.local) {
             if (rank == tb.endRank && d == tb.endLocal && pos == L && r >= 0) args.loglike[r] = sH;  // viterbi.h:102
@@ -824,7 +859,7 @@ __global__ void __launch_bounds__(W * 32, 1)
 }
 
 // ---------------------------------------------------------------------------
-// traceback over batch-layout records: one thread per read follows the predecessor bytes
+// traceback over batch-layout records: one thread per read follows the predecessor records
 // (reference src/viterbi.cpp:195-304: loop :247, emitted symbols :299-300), decoding each byte against the
 // state's transition lists in REFERENCE order (the records are indexed by reference state)
 // ---------------------------------------------------------------------------
@@ -876,6 +911,7 @@ __global__ void viterbiTracebackBatchKernel(const BatchTraceTables tb, const Bat
     return;
   }
   const uint8_t* predG = args.pred + (size_t)group * (size_t)(args.maxLen + 1) * N * K2 * 32 + lane;
+  const uint8_t* predWideG = args.predWide + (size_t)group * (size_t)(args.maxLen + 1) * tb.nWide * 64 + lane;
   int32_t pos = L;
   uint32_t mut = 0;
   const int32_t cap = args.decodedStride;
@@ -889,8 +925,16 @@ __global__ void viterbiTracebackBatchKernel(const BatchTraceTables tb, const Bat
         status = DNAB_READ_OVERFLOW_;
     }
     ++nPath;
-    const uint32_t p = predG[(((size_t)pos * N + state) * K2 + mut) * 32];
-    if (p == kNoPred) {
+    uint32_t p = predG[(((size_t)pos * N + state) * K2 + mut) * 32];
+    uint32_t none = kNoPred;
+    if (tb.wideOf && mut < 2) {  // a wide state's S and D records: the high byte is in the side plane
+      const uint32_t wn = tb.wideOf[state];
+      if (wn != 0xFFFFFFFFu) {
+        p |= (uint32_t)predWideG[(((size_t)pos * tb.nWide + wn) * 2 + mut) * 32] << 8;
+        none = kWideNoPred;
+      }
+    }
+    if (p == none) {
       status = DNAB_READ_TRACEBACK_FAILED_;
       break;
     }
@@ -948,18 +992,22 @@ __global__ void viterbiTracebackBatchKernel(const BatchTraceTables tb, const Bat
 // launchers
 // ---------------------------------------------------------------------------
 typedef void (*BatchKernelPtr)(const BatchTables, const BatchArgs);
-template <int W, int KMAX>
+template <int W, int KMAX, bool kWide>
 static BatchKernelPtr pickBatchKernelWK(bool team, bool debug) {
-  if (debug) return team ? viterbiFillBatchKernel<W, KMAX, true, true> : viterbiFillBatchKernel<W, KMAX, false, true>;
-  return team ? viterbiFillBatchKernel<W, KMAX, true, false> : viterbiFillBatchKernel<W, KMAX, false, false>;
+  if (debug) return team ? viterbiFillBatchKernel<W, KMAX, true, true, kWide> : viterbiFillBatchKernel<W, KMAX, false, true, kWide>;
+  return team ? viterbiFillBatchKernel<W, KMAX, true, false, kWide> : viterbiFillBatchKernel<W, KMAX, false, false, kWide>;
 }
 static uint32_t batchWarps(uint32_t warps) { return warps > 24 ? 32u : warps > 16 ? 24u : 16u; }
-static BatchKernelPtr pickBatchKernel(const BatchTables& tb, uint32_t warps, bool debug) {
+template <bool kWide>
+static BatchKernelPtr pickBatchKernelW(const BatchTables& tb, uint32_t warps, bool debug) {
   const bool team = tb.T > 1;
   const uint32_t w = batchWarps(warps);
-  if (w == 32) return tb.k <= 2 ? pickBatchKernelWK<32, 2>(team, debug) : pickBatchKernelWK<32, kMaxK>(team, debug);
-  if (w == 24) return tb.k <= 2 ? pickBatchKernelWK<24, 2>(team, debug) : pickBatchKernelWK<24, kMaxK>(team, debug);
-  return tb.k <= 2 ? pickBatchKernelWK<16, 2>(team, debug) : pickBatchKernelWK<16, kMaxK>(team, debug);
+  if (w == 32) return tb.k <= 2 ? pickBatchKernelWK<32, 2, kWide>(team, debug) : pickBatchKernelWK<32, kMaxK, kWide>(team, debug);
+  if (w == 24) return tb.k <= 2 ? pickBatchKernelWK<24, 2, kWide>(team, debug) : pickBatchKernelWK<24, kMaxK, kWide>(team, debug);
+  return tb.k <= 2 ? pickBatchKernelWK<16, 2, kWide>(team, debug) : pickBatchKernelWK<16, kMaxK, kWide>(team, debug);
+}
+static BatchKernelPtr pickBatchKernel(const BatchTables& tb, uint32_t warps, bool debug) {
+  return tb.nWide ? pickBatchKernelW<true>(tb, warps, debug) : pickBatchKernelW<false>(tb, warps, debug);
 }
 
 cudaError_t queryBatchTeams(const BatchTables& tb, uint32_t warps, uint32_t smemBytes, int* ctasPerSm) {

@@ -263,7 +263,8 @@ __device__ __forceinline__ uint32_t pushState(const Ctx& c, uint32_t s, uint4 sl
 
 }  // namespace
 
-template <int kMaxThreads, int kMinBlocks, bool kCluster, bool kDebug>
+// kWide: the machine has wide states (viterbi_device.cuh); only those machines run this instantiation.
+template <int kMaxThreads, int kMinBlocks, bool kCluster, bool kDebug, bool kWide>
 __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
     viterbiFillPushKernel(const __grid_constant__ DevTables tb, const __grid_constant__ FillArgs args) {
   constexpr int kU = kPushStatesPerThread;  // states per thread and step of a dense pass
@@ -468,6 +469,17 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
       };
       // record of slot u of this thread in the staged chunk, and its header (padding header when out of range)
       auto recOf = [&](uint32_t u) -> uint32_t { return aBuf + recBase + 4 * lds16(aBuf + 2 * (u * nThreads + tid)); };
+      // a wide state's record: its 16-bit counts and wide number follow the header; rec then points one header before
+      // its edges, like a narrow record's
+      auto wideRecord = [&](uint32_t h, uint32_t& rec, uint32_t& nIn, uint32_t& nE, uint32_t& wn) -> bool {
+        if (!kWide || inNIn(h) != kInWide) return false;
+        const uint32_t c2 = lds32(rec + 4);
+        nE = c2 & 0xFFFFu;
+        nIn = c2 >> 16;
+        wn = lds32(rec + 8);
+        rec += 8;
+        return true;
+      };
 
       // Duplication cells without storing them (k <= 2, S columns published in global scratch): T(p,1) =
       // (S(p)+tanDup)+len[1] and T(p,0) = max(T(p-1,1)+sub[ctx1][x_p], (S(p)+tanDup)+len[0]) are functions of
@@ -516,7 +528,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
       // when its new values can still raise a successor above what S0 / -inf already gave it.
       for (uint32_t j = 0; j < nChunks; ++j) {
         prefetch();
-        uint32_t i[kU], rec[kU], h[kU], nIn[kU];
+        uint32_t i[kU], rec[kU], h[kU], nIn[kU], nEw[kU], wn[kU];
         double s0[kU], newS[kU], newD[kU];
         uint32_t maxIn = 0;
 #pragma unroll
@@ -525,6 +537,8 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
           rec[u] = recOf(u);
           h[u] = i[u] < M ? lds32(rec[u]) : (kInPad << 7);
           nIn[u] = inNIn(h[u]) == kInPad ? 0u : inNIn(h[u]);
+          nEw[u] = inNEmit(h[u]);
+          wideRecord(h[u], rec[u], nIn[u], nEw[u], wn[u]);
           maxIn = max(maxIn, nIn[u]);
           s0[u] = i[u] < M ? ldsCell(aScur + 8 * i[u]) : NEG;
           newS[u] = s0[u];
@@ -543,7 +557,7 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
 #pragma unroll
           for (int u = 0; u < kU; ++u) {
             const double sc = ldsTab(aSym + 8 * peSym(w[u]));
-            if (e < inNEmit(h[u]))
+            if (e < (kWide ? nEw[u] : inNEmit(h[u])))
               newD[u] = dmax(newD[u], dmax(ds[u] + delExtend, ss[u] + delOpen) + sc);
             else if (e < nIn[u]) {
               newD[u] = dmax(newD[u], ds[u] + sc);
@@ -718,9 +732,11 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
       // ---- (3) predecessor records with the traceback's arithmetic (src/viterbi.cpp:251-286)
       //      (4) duplication opens (src/viterbi.cpp:161-168) ----
       uint8_t* predCol = predRead + (size_t)pos * (k + 2) * Np;
+      uint8_t* const predWideCol = kWide ? args.predWide + ((size_t)read * (args.maxLen + 1) + pos) * 2 * tb.nWide : nullptr;
       for (uint32_t j = 0; j < nChunks; ++j) {
         prefetch();
-        uint32_t i[kU], rec[kU], h[kU], nIn[kU], idx[kU], idxD[kU];
+        uint32_t i[kU], rec[kU], h[kU], nIn[kU], idx[kU], idxD[kU], nEw[kU], wn[kU];
+        bool wide[kU];
         double sHere[kU], dHere[kU], parked[kU], tPrev1[kU], best[kU], bestD[kU], s0n[kU];
         uint32_t maxIn = 0;
 #pragma unroll
@@ -729,6 +745,8 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
           rec[u] = recOf(u);
           h[u] = i[u] < M ? lds32(rec[u]) : (kInPad << 7);
           nIn[u] = inNIn(h[u]) == kInPad ? 0u : inNIn(h[u]);
+          nEw[u] = inNEmit(h[u]);
+          wide[u] = wideRecord(h[u], rec[u], nIn[u], nEw[u], wn[u]);
           maxIn = max(maxIn, nIn[u]);
           const uint32_t mdl = inMdl(h[u]);
           sHere[u] = i[u] < M ? ldsCell(aScur + 8 * i[u]) : NEG;
@@ -742,8 +760,8 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
             parked[u] = (mdl > 0 && pos > 0) ? tCol[(mdl - 1) * M + i[u]] : NEG;  // T(state,pos-1,0)+sub
           best[u] = NEG;
           bestD[u] = NEG;
-          idx[u] = kNoPred;
-          idxD[u] = kNoPred;
+          idx[u] = wide[u] ? kWideNoPred : kNoPred;
+          idxD[u] = idx[u];
           s0n[u] = NEG;
         }
         for (uint32_t e = 0; e < maxIn; ++e) {
@@ -755,11 +773,11 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
           for (int u = 0; u < kU; ++u) {
             vs[u] = e < nIn[u] ? loadCell(aScur, w[u]) : NEG;
             vd[u] = e < nIn[u] ? loadCell(aD, w[u]) : NEG;
-            vp[u] = (pos > 0 && e < inNEmit(h[u])) ? loadPrev(w[u]) : NEG;
+            vp[u] = (pos > 0 && e < (kWide ? nEw[u] : inNEmit(h[u]))) ? loadPrev(w[u]) : NEG;
           }
 #pragma unroll
           for (int u = 0; u < kU; ++u) {
-            const uint32_t nE = inNEmit(h[u]);
+            const uint32_t nE = kWide ? nEw[u] : inNEmit(h[u]);
             const uint32_t sym8 = 8 * peSym(w[u]);
             if (e < nE) {
               if (pos > 0) {
@@ -825,6 +843,10 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
             }
             predCol[g] = (uint8_t)(real ? idx[u] : kNoPred);
             predCol[Np + g] = (uint8_t)(real ? idxD[u] : kNoPred);
+            if (wide[u]) {  // the high bytes (a wide state is real)
+              predWideCol[wn[u]] = (uint8_t)(idx[u] >> 8);
+              predWideCol[tb.nWide + wn[u]] = (uint8_t)(idxD[u] >> 8);
+            }
             double* cell = (kDebug && args.cells && read == 0 && real)  // the cell dump exists in the kDebug kernel only
                                ? args.cells + ((size_t)pos * tb.nStates + __ldg(&tb.origId[g])) * (k + 2)
                                : nullptr;
@@ -938,22 +960,26 @@ __global__ void __launch_bounds__(kMaxThreads, kMinBlocks)
 // launchers
 // ---------------------------------------------------------------------------
 typedef void (*PushKernelPtr)(const DevTables, const FillArgs);
-template <bool kCluster, bool kDebug>
+template <bool kCluster, bool kDebug, bool kWide>
 static PushKernelPtr pickPushKernelT(uint32_t threads) {
-  if (threads > 800) return viterbiFillPushKernel<1024, 1, kCluster, kDebug>;  // 64 registers/thread
-  if (threads > 640) return viterbiFillPushKernel<800, 1, kCluster, kDebug>;   // 80
-  if (threads > 512) return viterbiFillPushKernel<640, 1, kCluster, kDebug>;   // 96
-  if (threads > 256) return viterbiFillPushKernel<512, 1, kCluster, kDebug>;   // 128
+  if (threads > 800) return viterbiFillPushKernel<1024, 1, kCluster, kDebug, kWide>;  // 64 registers/thread
+  if (threads > 640) return viterbiFillPushKernel<800, 1, kCluster, kDebug, kWide>;   // 80
+  if (threads > 512) return viterbiFillPushKernel<640, 1, kCluster, kDebug, kWide>;   // 96
+  if (threads > 256) return viterbiFillPushKernel<512, 1, kCluster, kDebug, kWide>;   // 128
   // narrow CTAs (small machines, many CTAs per SM): registers are allocated in units of 8, so 81 means 88 and one
   // resident CTA fewer than 80 -- a third block in the launch bounds caps the one-CTA kernel at 80
   if constexpr (!kCluster)
-    return viterbiFillPushKernel<256, 3, false, kDebug>;  // 80
+    return viterbiFillPushKernel<256, 3, false, kDebug, kWide>;  // 80
   else
-    return viterbiFillPushKernel<256, 2, true, kDebug>;  // 128
+    return viterbiFillPushKernel<256, 2, true, kDebug, kWide>;  // 128
+}
+template <bool kWide>
+static PushKernelPtr pickPushKernelW(const DevTables& tb, uint32_t threads, bool debug) {
+  if (debug) return tb.C > 1 ? pickPushKernelT<true, true, kWide>(threads) : pickPushKernelT<false, true, kWide>(threads);
+  return tb.C > 1 ? pickPushKernelT<true, false, kWide>(threads) : pickPushKernelT<false, false, kWide>(threads);
 }
 static PushKernelPtr pickPushKernel(const DevTables& tb, uint32_t threads, bool debug) {
-  if (debug) return tb.C > 1 ? pickPushKernelT<true, true>(threads) : pickPushKernelT<false, true>(threads);
-  return tb.C > 1 ? pickPushKernelT<true, false>(threads) : pickPushKernelT<false, false>(threads);
+  return tb.nWide ? pickPushKernelW<true>(tb, threads, debug) : pickPushKernelW<false>(tb, threads, debug);
 }
 
 static cudaError_t prepPush(PushKernelPtr kern, const DevTables& tb, uint32_t smemBytes) {

@@ -91,7 +91,8 @@ struct FillArgs {
   const int64_t* byteOff;    // [nReads]
   const int32_t* readLen;    // [nReads]
   uint8_t* pred;             // [nReads][maxLen+1][k+2][Np] predecessor records, 1 byte per DP cell
-  double* tScratch;          // [nClusters*C][k][M] T columns when they do not fit in shared memory
+  uint8_t* predWide;         // [nReads][maxLen+1][2][nWide] high bytes of the wide states' S and D records (viterbi_device.cuh)
+  double* tScratch;         // [nClusters*C][k][M] T columns when they do not fit in shared memory
   double* sScratch;          // [nClusters][2][Np] S columns of the last two positions when S(pos-1) is not in shared memory
   double* s0Scratch;         // [nClusters][Np] S0 of the next column (the emission step is fused into the predecessor pass)
   double* loglike;           // [nReads] (global mode; local mode: written by the traceback kernel)
@@ -109,6 +110,7 @@ struct TracebackArgs {
   int32_t maxLen;
   const int32_t* readLen;
   const uint8_t* pred;
+  const uint8_t* predWide;
   double* loglike;
   const uint32_t* startState;
   const double* partVal;

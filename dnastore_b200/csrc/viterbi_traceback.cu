@@ -1,10 +1,10 @@
 // viterbiTracebackKernel: the traceback of the Viterbi fill (reference src/viterbi.cpp:195-304) for the
 // one-read-per-cluster push kernel (viterbi_fill_push.cu), on the device, one thread per read.
 //
-// The fill leaves one predecessor byte per DP cell, evaluated with the traceback's own floating-point
-// association and candidate order; this kernel follows those bytes from the end cell back to the start
-// state and decodes each byte against the state blocks (viterbi_device.cuh) that the host built for the
-// same partition.  It writes the decoded input-symbol string, the log-likelihood (local mode: the best
+// The fill leaves one predecessor byte per DP cell (two for the S and D cells of wide states, the high
+// byte in the side plane), evaluated with the traceback's own floating-point association and candidate
+// order; this kernel follows those records from the end cell back to the start state and decodes each
+// against the state blocks (viterbi_device.cuh) that the host built for the same partition.  It writes the decoded input-symbol string, the log-likelihood (local mode: the best
 // of the per-CTA maxima the fill left) and the status of every read, and optionally the path of cells.
 #include <cuda_runtime.h>
 
@@ -73,14 +73,24 @@ __global__ void viterbiTracebackKernel(const DevTables tb, const TracebackArgs a
         status = DNAB_READ_OVERFLOW_;
     }
     ++nPath;
-    const uint32_t p = predRead[((size_t)pos * (k + 2) + mut) * Np + g];
-    if (p == kNoPred) {
+    uint32_t p = predRead[((size_t)pos * (k + 2) + mut) * Np + g];
+    const uint32_t* blkp = tb.blocks + tb.blockOff[g];
+    uint32_t nE = hdrNEmit(blkp[0]), nIn = hdrNIn(blkp[0]);
+    const uint2* edges = reinterpret_cast<const uint2*>(blkp + 2);
+    uint32_t none = kNoPred;
+    if (nE == kHdrWide) {  // wide state: 16-bit counts, and the S and D records' high bytes in the side plane
+      nE = blkp[2] & 0xFFFFu;
+      nIn = blkp[2] >> 16;
+      edges = reinterpret_cast<const uint2*>(blkp + 4);
+      if (mut < 2) {
+        p |= (uint32_t)args.predWide[((size_t)read * (args.maxLen + 1) + pos) * 2 * tb.nWide + mut * tb.nWide + blkp[3]] << 8;
+        none = kWideNoPred;
+      }
+    }
+    if (p == none) {
       status = DNAB_READ_TRACEBACK_FAILED_;
       break;
     }
-    const uint32_t* blkp = tb.blocks + tb.blockOff[g];
-    const uint32_t nE = hdrNEmit(blkp[0]), nIn = hdrNIn(blkp[0]);
-    const uint2* edges = reinterpret_cast<const uint2*>(blkp + 2);
     auto srcOf = [&](uint2 e) { return edgeRank(e.x) * M + edgeOff(e.x) / 8; };
     uint32_t sym = 0;
     if (mut == 0) {

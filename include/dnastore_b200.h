@@ -156,7 +156,7 @@ typedef struct dnab_batch_info {
   uint32_t warps_per_cta;
   uint32_t smem_bytes_per_cta;
   uint32_t n_teams;            /* groups in flight */
-  uint32_t reserved;
+  uint32_t wide_states;        /* wide states of the machine (see dnab_viterbi_batch); 0 = no side plane */
   double cross_cta_transition_fraction; /* transitions whose source and destination live in different CTAs */
 } dnab_batch_info;
 int dnab_decoder_get_batch_info(const dnab_decoder* d, dnab_batch_info* info);
@@ -183,7 +183,18 @@ int dnab_pack_reads(const char* bases, const int64_t* base_off, int64_t n_reads,
  *                       (state, pos, mutState) with mutState 0=S,1=D,2+i=T(i+1)
  *                       (src/viterbi.h:52-56), in traceback order starting at the
  *                       first cell the reference's loop visits; path_stride triples per read
- * Returns DNAB_OK or a negative code. */
+ * Returns DNAB_OK or a negative code.
+ *
+ * Viterbi decoding takes states of any in- and out-degree that the reference accepts.  The predecessor
+ * record of a DP cell is one byte; a state with more candidates than a byte can name, or with more
+ * than 255 outgoing transitions, is a WIDE state (nEmit > 126, nEmit + nNull + 2 > 254, 2*nEmit + nNull
+ * > 254, or > 255 outgoing transitions): the high byte of its S and D records goes to a side plane
+ * sized nWide * 2 bytes per read and column, allocated only for machines that have wide states
+ * (dnab_batch_info.wide_states counts them).  Still refused with DNAB_EINVAL, the state named in the
+ * error text: a state with more than 65,535 candidates in a record (nEmit + nNull + 3 or
+ * 2*nEmit + nNull > 65,535: a wide record is 16 bits, 0xFFFF = none), or with more than 65,535
+ * outgoing transitions.  Independently of degree, the tables of one CTA use 16-bit offsets; a
+ * machine whose tables exceed them for every placement is refused as not fitting. */
 int dnab_viterbi_batch(dnab_decoder* d, int64_t n_reads, const uint8_t* packed, const int64_t* read_byte_off,
                        const int32_t* read_len, double* loglike, char* decoded, int32_t decoded_stride,
                        int32_t* decoded_len, int32_t* status, int32_t* path, int32_t path_stride, int32_t* path_len);
