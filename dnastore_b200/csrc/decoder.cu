@@ -1085,11 +1085,11 @@ static cudaError_t takeEvents(dnab_decoder* d, bool timeIt, cudaEvent_t ev[3], b
   return cudaSuccess;
 }
 
-// fill + traceback with the read-batched kernel; hostLen (optional) lets the groups be formed from reads of similar length
+// fill + traceback with the read-batched kernel
 static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint8_t* dPacked, const int64_t* dByteOff,
                           const int32_t* dReadLen, double* dLoglike, char* dDecoded, int32_t decodedStride,
                           int32_t* dDecodedLen, int32_t* dStatus, int32_t* dPath, int32_t pathStride, int32_t* dPathLen,
-                          double* dCells, cudaStream_t stream, bool timeIt, const int32_t* hostLen) {
+                          double* dCells, cudaStream_t stream, bool timeIt) {
   const BatchPlan& bp = d->bplan;
   const uint32_t N = d->nStates, K2 = d->k + 2;
   const int64_t nGroups = (nReads + 31) / 32;
@@ -1104,14 +1104,13 @@ static int runDeviceBatch(dnab_decoder* d, int64_t nReads, int32_t maxLen, const
     CUDA_TRY(d->dbPartOrig.ensure((size_t)chunk * bp.T * bp.warps * 32));
   }
   const int32_t* dOrder = nullptr;
-  if (hostLen && !dCells && nReads > 32) {
-    // groups of similar length: a group runs for as many columns as its longest read
-    std::vector<int32_t> order((size_t)nGroups * 32, -1);
-    for (int64_t i = 0; i < nReads; ++i) order[(size_t)i] = (int32_t)i;
-    std::stable_sort(order.begin(), order.begin() + nReads, [&](int32_t a, int32_t b) { return hostLen[a] > hostLen[b]; });
-    CUDA_TRY(d->dbOrder.ensure(order.size()));
-    CUDA_TRY(cudaMemcpyAsync(d->dbOrder.p, order.data(), order.size() * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
-    CUDA_TRY(cudaStreamSynchronize(stream));  // `order` is a local
+  if (!dCells && nReads > 32) {
+    // groups of similar length, formed on the device from dReadLen: a group runs for as many columns as its longest read
+    const size_t nSlots = (size_t)nGroups * 32;
+    CUDA_TRY(d->dbOrder.ensure(nSlots + (size_t)maxLen + 1));  // the order, then the sort's bins
+    CUDA_TRY(launchLengthOrder(dReadLen, nReads, maxLen, (int64_t)nSlots, d->dbOrder.p,
+                               reinterpret_cast<uint32_t*>(d->dbOrder.p + nSlots), stream));
+    d->stats.kernel_launches += 1;
     dOrder = d->dbOrder.p;
   }
   for (int64_t at = 0; at < nGroups; at += chunk) {
@@ -1192,7 +1191,7 @@ static size_t predWideBytesPerRead(const dnab_decoder* d, int32_t maxLen) { retu
 static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint8_t* dPacked, const int64_t* dByteOff,
                      const int32_t* dReadLen, double* dLoglike, char* dDecoded, int32_t decodedStride,
                      int32_t* dDecodedLen, int32_t* dStatus, int32_t* dPath, int32_t pathStride, int32_t* dPathLen,
-                     double* dCells, cudaStream_t stream, bool timeIt, const int32_t* hostLen = nullptr) {
+                     double* dCells, cudaStream_t stream, bool timeIt) {
   if (nReads <= 0) return DNAB_OK;
   CUDA_TRY(cudaSetDevice(d->device));
   if (batchWanted(d)) {
@@ -1206,7 +1205,7 @@ static int runDevice(dnab_decoder* d, int64_t nReads, int32_t maxLen, const uint
     if (use && d->wantBatch != 1 && d->bplan.T > 1 && buildPlan(d, maxLen) == DNAB_OK && d->plan.C < 4) use = false;
     if (use)
       return runDeviceBatch(d, nReads, maxLen, dPacked, dByteOff, dReadLen, dLoglike, dDecoded, decodedStride, dDecodedLen,
-                            dStatus, dPath, pathStride, dPathLen, dCells, stream, timeIt, hostLen);
+                            dStatus, dPath, pathStride, dPathLen, dCells, stream, timeIt);
     if (d->wantBatch == 1) return brc;
   }
   int rc = buildPlan(d, maxLen);
@@ -1617,7 +1616,7 @@ static int viterbiHost(dnab_decoder* d, int64_t n, const uint8_t* packed, const 
   CUDA_TRY(cudaMemcpyAsync(d->dReadLen.p, readLen, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, stream));
   int rc = runDevice(d, n, maxLen, d->dPacked.p, d->dByteOff.p, d->dReadLen.p, d->dLoglike.p, d->dDecoded.p, decodedStride,
                      d->dDecodedLen.p, d->dStatus.p, path ? d->dPath.p : nullptr, pathStride,
-                     path ? d->dPathLen.p : nullptr, cells ? d->dCells.p : nullptr, stream, true, readLen);
+                     path ? d->dPathLen.p : nullptr, cells ? d->dCells.p : nullptr, stream, true);
   if (rc != DNAB_OK) return rc;
   CUDA_TRY(cudaMemcpyAsync(loglike, d->dLoglike.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, stream));
   CUDA_TRY(cudaMemcpyAsync(decoded, d->dDecoded.p, (size_t)n * decodedStride, cudaMemcpyDeviceToHost, stream));

@@ -198,5 +198,8 @@ cudaError_t queryBatchTeams(const BatchTables& tb, uint32_t warps, uint32_t smem
 cudaError_t launchFillBatch(const BatchTables& tb, const BatchArgs& args, uint32_t warps, uint32_t smemBytes,
                             cudaStream_t stream, size_t persistBytes);
 cudaError_t launchTracebackBatch(const BatchTraceTables& tb, const BatchTraceArgs& args, cudaStream_t stream);
+// order[0, nSlots): the reads by descending length, ties in input order, then -1; bins: maxLen + 1 words of scratch
+cudaError_t launchLengthOrder(const int32_t* readLen, int64_t nReads, int32_t maxLen, int64_t nSlots, int32_t* order,
+                              uint32_t* bins, cudaStream_t stream);
 
 }  // namespace dnab

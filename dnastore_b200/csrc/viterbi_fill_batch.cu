@@ -989,6 +989,63 @@ __global__ void viterbiTracebackBatchKernel(const BatchTraceTables tb, const Bat
 }
 
 // ---------------------------------------------------------------------------
+// slot -> read order of the groups: reads by descending length, ties in input order (a stable counting sort
+// over the lengths in [0, maxLen]), so that a group runs for about as many columns as each of its reads
+// needs.  One CTA: a histogram, an exclusive scan over the bins, then warp 0 deals the reads out 32 at a
+// time in input order, which is what keeps the sort stable.
+// ---------------------------------------------------------------------------
+constexpr int kOrderThreads = 1024;
+
+__global__ void __launch_bounds__(kOrderThreads, 1)
+    lengthOrderKernel(const int32_t* readLen, int32_t nReads, int32_t maxLen, int64_t nSlots, int32_t* order,
+                      uint32_t* bins) {
+  __shared__ uint32_t part[kOrderThreads];
+  const uint32_t tid = threadIdx.x, lane = tid & 31u, nBins = (uint32_t)maxLen + 1u;
+  // bin of a read: longest first; a length outside [0, maxLen] is clamped so that it cannot index past the bins
+  auto binOf = [&](int32_t r) { return (uint32_t)(maxLen - min(max(readLen[r], 0), maxLen)); };
+  for (uint32_t b = tid; b < nBins; b += kOrderThreads) bins[b] = 0;
+  for (int64_t s = nReads + tid; s < nSlots; s += kOrderThreads) order[s] = -1;
+  __syncthreads();
+  for (int32_t r = tid; r < nReads; r += kOrderThreads) atomicAdd(bins + binOf(r), 1u);
+  __syncthreads();
+  // exclusive scan: thread t owns bins [t*per, (t+1)*per)
+  const uint32_t per = (nBins + kOrderThreads - 1) / kOrderThreads, lo = min(tid * per, nBins), hi = min(lo + per, nBins);
+  uint32_t sum = 0;
+  for (uint32_t b = lo; b < hi; ++b) sum += bins[b];
+  part[tid] = sum;
+  __syncthreads();
+  for (uint32_t d = 1; d < kOrderThreads; d <<= 1) {
+    const uint32_t add = tid >= d ? part[tid - d] : 0u;
+    __syncthreads();
+    part[tid] += add;
+    __syncthreads();
+  }
+  uint32_t at = part[tid] - sum;
+  for (uint32_t b = lo; b < hi; ++b) {
+    const uint32_t c = bins[b];
+    bins[b] = at;
+    at += c;
+  }
+  __syncthreads();
+  if (tid >= 32) return;
+  for (int32_t base = 0; base < nReads; base += 32) {
+    const int32_t r = base + (int32_t)lane;
+    const uint32_t b = r < nReads ? binOf(r) : 0xFFFFFFFFu;
+    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, b), first = __ffs(peers) - 1;
+    uint32_t slot = 0;
+    if (lane == first && r < nReads) slot = atomicAdd(bins + b, (uint32_t)__popc(peers));
+    slot = __shfl_sync(0xFFFFFFFFu, slot, first) + __popc(peers & ((1u << lane) - 1u));
+    if (r < nReads) order[slot] = r;
+  }
+}
+
+cudaError_t launchLengthOrder(const int32_t* readLen, int64_t nReads, int32_t maxLen, int64_t nSlots, int32_t* order,
+                              uint32_t* bins, cudaStream_t stream) {
+  lengthOrderKernel<<<1, kOrderThreads, 0, stream>>>(readLen, (int32_t)nReads, maxLen, nSlots, order, bins);
+  return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------
 typedef void (*BatchKernelPtr)(const BatchTables, const BatchArgs);
