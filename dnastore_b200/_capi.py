@@ -71,7 +71,8 @@ class PipelineStats(C.Structure):
 class DecoderStats(C.Structure):
     _fields_ = [("kernel_launches", C.c_uint64), ("fill_launches", C.c_uint64), ("traceback_launches", C.c_uint64),
                 ("reads", C.c_uint64), ("cells", C.c_uint64), ("last_fill_ms", C.c_double), ("last_traceback_ms", C.c_double),
-                ("timed_fill_ms", C.c_double), ("timed_traceback_ms", C.c_double), ("timed_fill_launches", C.c_uint64)]
+                ("timed_fill_ms", C.c_double), ("timed_traceback_ms", C.c_double), ("timed_fill_launches", C.c_uint64),
+                ("last_fwd_threads", C.c_uint32), ("last_fwd_blocks", C.c_uint32)]
 
 
 class MutatorParams(C.Structure):

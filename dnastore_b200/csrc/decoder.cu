@@ -103,6 +103,8 @@ struct dnab_decoder {
   DevBuf<unsigned long long> dDbg, dNextRead;
   // forward kernel (forward_kernels.cu): CSR tables in reference order, uploaded on first use
   bool fwdReady = false;
+  uint32_t fwdThreads = 0;  // options "fwd_threads" (CTA width, 0 = by state count) and "fwd_blocks" (grid cap, 0 = none)
+  uint32_t fwdBlocks = 0;
   DevBuf<uint32_t> dFwdEmitOff, dFwdEmitSrc, dFwdNullOff, dFwdNullSrc;
   DevBuf<uint8_t> dFwdEmitMeta, dFwdNullSym, dFwdCtx, dFwdMdl;
   DevBuf<double> dFwdLse, dFwdScratch, dFwdF, dFwdCounts, dFwdLLBack;
@@ -1460,7 +1462,19 @@ int dnab_decoder_set_option(dnab_decoder* d, const char* key, int64_t value) {
     d->wantPersist = v;
   else if (k == "pred_budget_mb")
     d->predBudgetBytes = (size_t)value << 20;
-  else {
+  else if (k == "fwd_threads") {
+    if (value != 0 && (value > 1024 || value % 32 != 0)) {
+      setLastError("dnab_decoder_set_option: fwd_threads must be 0 (automatic) or a multiple of 32 from 32 to 1024");
+      return DNAB_EINVAL;
+    }
+    d->fwdThreads = v;
+  } else if (k == "fwd_blocks") {
+    if (value > UINT32_MAX) {
+      setLastError("dnab_decoder_set_option: fwd_blocks must be below 2^32");
+      return DNAB_EINVAL;
+    }
+    d->fwdBlocks = v;
+  } else {
     setLastError("dnab_decoder_set_option: unknown option '" + k + "'");
     return DNAB_EINVAL;
   }
@@ -1718,7 +1732,7 @@ static int forwardImpl(dnab_decoder* d, int64_t n, const uint8_t* packed, const 
   packedBytes = std::max<size_t>(packedBytes, 16);
   // one CTA per read in flight; small machines get narrower CTAs and several of them per SM (the kernel is capped
   // at 64 registers, so 1024 threads per SM in total): l4c4 (384 states) 12.1k -> 24.0k reads/s
-  const uint32_t fwdThreads = N >= 4096 ? 1024u : N >= 2048 ? 512u : N >= 1024 ? 256u : 128u;
+  const uint32_t fwdThreads = d->fwdThreads ? d->fwdThreads : N >= 4096 ? 1024u : N >= 2048 ? 512u : N >= 1024 ? 256u : 128u;
   const uint32_t fwdPerSm = 1024 / fwdThreads;
   uint32_t nBlocks = (uint32_t)std::min<int64_t>(n, (int64_t)d->smCount * fwdPerSm);
   const uint32_t nc = 5 + k + 16;
@@ -1728,6 +1742,9 @@ static int forwardImpl(dnab_decoder* d, int64_t n, const uint8_t* packed, const 
     cudaMemGetInfo(&freeB, &totalB);
     const size_t budget = std::max<size_t>(d->dFwdF.n * sizeof(double), freeB / 2);
     nBlocks = (uint32_t)std::max<size_t>(1, std::min<size_t>(nBlocks, budget / (fPerBlock * sizeof(double))));
+  }
+  if (d->fwdBlocks) nBlocks = std::min(nBlocks, d->fwdBlocks);
+  if (counts) {
     CUDA_TRY(d->dFwdF.ensure((size_t)nBlocks * fPerBlock));
     CUDA_TRY(d->dFwdCounts.ensure((size_t)n * nc));
     CUDA_TRY(d->dFwdLLBack.ensure((size_t)n));
@@ -1815,6 +1832,8 @@ static int forwardImpl(dnab_decoder* d, int64_t n, const uint8_t* packed, const 
   CUDA_TRY(launchForward(ft, fa, nBlocks, fwdThreads, stream));
   CUDA_TRY(cudaEventRecord(d->ev1, stream));
   d->stats.kernel_launches += 1;
+  d->stats.last_fwd_threads = fwdThreads;
+  d->stats.last_fwd_blocks = nBlocks;
   CUDA_TRY(cudaMemcpyAsync(loglike, d->dLoglike.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, stream));
   std::vector<long long> sw(sweeps ? (size_t)n : 0);
   if (sweeps) CUDA_TRY(cudaMemcpyAsync(sw.data(), d->dFwdSweeps.p, (size_t)n * sizeof(long long), cudaMemcpyDeviceToHost, stream));
@@ -1850,7 +1869,8 @@ int dnab_posterior_classes(const dnab_decoder* d, char* classes, size_t cap) {
   if (!d || !classes) return DNAB_EINVAL;
   const size_t n = d->symChar.size() + 1;
   if (n > (size_t)kPostClasses) {
-    setLastError("posterior decoding tells at most " + std::to_string(kPostClasses - 1) + " input symbols apart; this machine has " +
+    // classes: "no input symbol", one per input symbol, "duplication"
+    setLastError("posterior decoding tells at most " + std::to_string(kPostClasses - 2) + " input symbols apart; this machine has " +
                  std::to_string(d->symChar.size() - 1));
     return DNAB_EINVAL;
   }

@@ -145,6 +145,15 @@ int dnab_decoder_configure(dnab_decoder* d, uint32_t cluster_size, uint32_t thre
  *   "persist_l2"      read-batched kernel: 1 gives the rows carried between columns a persisting L2 access-policy window (default 0:
  *                     measured on B200 it DOUBLES the DRAM writes; the rows carry an evict-last cache hint instead)
  *   "pred_budget_mb"  device memory the predecessor records of one launch may take
+ *   "fwd_threads"     forward-family kernel (dnab_forward_batch, dnab_fwdback_counts_batch, dnab_posterior_batch): threads
+ *                     per CTA, a multiple of 32 from 32 to 1024 (anything else is DNAB_EINVAL); 0 (default) chooses from the
+ *                     state count: 128, 256, 512 or 1024 threads from 1024, 2048 and 4096 states up.  A CTA evaluates only
+ *                     the frontier of a sweep when the machine has at least 4 states per thread
+ *   "fwd_blocks"      forward-family kernel: at most this many CTAs (0 = default: up to 1024 threads per SM, one read per
+ *                     CTA in flight, fewer when the forward cells kept for the backward pass would exceed half the free
+ *                     device memory); 1 runs the whole batch through one CTA, read after read.
+ *                     Neither option changes a result bit for bit except the counts and posteriors, whose sums over the
+ *                     states run in an order fixed by the CTA width (equal to 1e-9 relative across widths)
  * Unknown keys return DNAB_EINVAL. */
 int dnab_decoder_set_option(dnab_decoder* d, const char* key, int64_t value);
 
@@ -245,7 +254,8 @@ int dnab_fwdback_counts_batch(dnab_decoder* d, int64_t n_reads, const uint8_t* p
  *   class 0        a transition that consumes no input symbol (padding / control-word bases)
  *   class 1..s     a transition that consumes input symbol classes[i] ('0', '1', control letters, ...)
  *   class s+1      a tandem duplication (the base repeats an earlier one, src/viterbi.cpp:102-106)
- * dnab_posterior_classes writes the class characters ("-" + the machine's input symbols + "+") and returns their number.
+ * dnab_posterior_classes writes the class characters ("-" + the machine's input symbols + "+") and returns their number;
+ * at most 8 classes, so a machine with more than 6 input symbols is refused with DNAB_EINVAL.
  * post: row post_off[r] + p, column c = P(class c emitted base p of read r | read); every row sums to 1 up to the accuracy
  * of the reference's table log_sum_exp (2e-3).  decoded (optional, one char per base, same offsets): the most probable
  * class per base -- a soft output for an outer code (doc/trans.tex:947-952,1148-1154), not the Viterbi input string.
@@ -269,6 +279,10 @@ typedef struct dnab_decoder_stats {
   double timed_fill_ms;
   double timed_traceback_ms;
   uint64_t timed_fill_launches;
+  /* launch shape of the most recent forward-family kernel (dnab_forward_batch, dnab_fwdback_counts_batch,
+   * dnab_posterior_batch): threads per CTA and CTAs in the grid */
+  uint32_t last_fwd_threads;
+  uint32_t last_fwd_blocks;
 } dnab_decoder_stats;
 /* Resolves pending timing events: call only after the stream(s) used have been synchronised. */
 int dnab_decoder_get_stats(const dnab_decoder* d, dnab_decoder_stats* s);
